@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the FFC head hot path (BASELINE.json metric: head fwd+bwd samples/s, % of bf16 tensor peak).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c4] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c4] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one reference ``FFC.forward`` over one synthetic batch, embeddings in: a rollback head pass
 (probe=x, gallery=y) plus a commit head pass (probe=y, gallery=x) -- ffc.py:264-267 -- i.e. 2*B probe rows
@@ -135,9 +135,8 @@ def cpu_head_runner(ws):
     return 'port', step
 
 
-def time_cpu(ws, steps, warmup, seed=1234, budget_s=60.0):
-    """Mean seconds per step over up to `steps` timed steps; stops early (after >= 2) once `budget_s` of timed work is spent, so that
-    the CPU arm ends within minutes whatever --steps says."""
+def time_cpu(ws, steps, warmup, seed=1234):
+    """Mean seconds per step over `steps` timed steps."""
     kind, step = cpu_head_runner(ws)
     batches = make_batches(ws, min(4, steps + warmup), seed=seed)
     times = []
@@ -148,8 +147,6 @@ def time_cpu(ws, steps, warmup, seed=1234, budget_s=60.0):
         dt = time.perf_counter() - t0
         if s >= warmup:
             times.append(dt)
-            if len(times) >= 2 and sum(times) > budget_s:
-                break
     return kind, sum(times) / len(times)
 
 
@@ -203,7 +200,7 @@ def run_reference(args, w):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
         return
-    cb, t = cpu_reference(w, max(1, args.steps), max(0, args.warmup))
+    cb, t = cpu_reference(w, args.steps, args.warmup)
     cfg = dict(config_of(w, max(1, args.gpus)),
                reference_sample=dict(rows_per_pass=cb['sample_rows_per_pass'], queue=cb['sample_queue'], extrapolated=cb['extrapolated'],
                                      rule='samples/s measured on the sample, multiplied by sample queue / full queue (cost per sample is linear in the queue size)'))
@@ -355,6 +352,17 @@ def softmax_rows(head, rows):
     return min(rows, (n_soft + 127) // 128 * 128)
 
 
+def dump_outputs(out_dir, out, rank, world):
+    """Write what the last timed step returned -- the loss and dLoss/dx, dLoss/dy ([B, D]) -- as float32 out_dir/<name>.npy (a rank
+    suffix when sharded), so that two builds of the project can be compared output for output.  At most 4 MB per rank (B = 1024,
+    D = 512)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = '' if world == 1 else f'_rank{rank}'
+    for name, t in zip(('loss', 'dx', 'dy'), out):
+        np.save(os.path.join(out_dir, f'{name}{suffix}.npy'), t.detach().float().cpu().numpy())
+
+
 def run_ours(args, w):
     import torch
     import torch.distributed as dist
@@ -371,6 +379,9 @@ def run_ours(args, w):
         dist.init_process_group('nccl', device_id=dev)
     lib = _capi.lib()
     B, N, Q, D = w['B'], w['N'], w['Q'], w['D']
+    # the initial queue (each rank's shard of it) is drawn from torch's global generators, which torch seeds differently in every
+    # process: seed them, so that every run with the same arguments (and every build of the project) starts from the same queue
+    torch.manual_seed(1234 + rank)
 
     if world == 1:
         head = ffc_b200.FFCHead(D, Q, w['scale'], w['loss_type'], w['margin'], precision='bf16', max_batch=B, device=dev)
@@ -378,8 +389,8 @@ def run_ours(args, w):
         # steady state: LRU full (SURVEY 8(d)): ids 0..Q-1 resident, slot i <- id i, recency = id order
         head.lru.restore_arrays(torch.arange(Q, dtype=torch.int64), torch.arange(Q, dtype=torch.int32))
 
-        def step(x, y, xl, yl):          # rollback pass (probe x, gallery y) + commit pass (probe y, gallery x): loss and both dEmb
-            return head.forward_pair(x, y, y, x, xl, yl)[0]
+        def step(x, y, xl, yl):          # rollback pass (probe x, gallery y) + commit pass (probe y, gallery x): (loss, dLoss/dx, dLoss/dy)
+            return head.forward_pair(x, y, y, x, xl, yl)
 
         def step_api(x, y, xl, yl):      # public API (FFC.forward with embeddings in), gradients requested
             return head(x.requires_grad_(True), y.requires_grad_(True), xl, yl)
@@ -389,9 +400,11 @@ def run_ours(args, w):
         head = ShardedFFCHead(D, Q, w['scale'], w['loss_type'], w['margin'], max_batch=B, device=dev)
         head.prefill_identity(N)
 
-        def step(x, y, xl, yl):
-            return head.forward_pair(x, y, xl, yl)[0]
-        step_api = step
+        def step(x, y, xl, yl):          # (loss, dLoss/dx, dLoss/dy) of this rank's rows
+            return head.forward_pair(x, y, xl, yl)
+
+        def step_api(x, y, xl, yl):
+            return step(x, y, xl, yl)[0]
         # the sharded head takes the NEXT step's labels (CPU tensors, main.py:59-60) as soon as the loader has them:
         # their all-gather and the rollback pass's LRU bookkeeping then run under the current step's sweeps
         prefetch = None if os.environ.get('FFC_BENCH_NO_PREFETCH') else head.prefetch
@@ -424,7 +437,7 @@ def run_ours(args, w):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for s in range(args.steps):
-        loss = step(*devb[(args.warmup + s) % n_b])
+        out = step(*devb[(args.warmup + s) % n_b])
         if prefetch and s + 1 < args.steps:
             prefetch(*devb[(args.warmup + s + 1) % n_b][2:])
     e1.record()
@@ -434,7 +447,9 @@ def run_ours(args, w):
     sweep_ms, sweep_n = head.get_timing()
     head.set_timing(False)
     clk = clocks.stop() if clocks else None
-    loss_val = float(loss)
+    loss_val = float(out[0])
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, rank, world)
 
     # ---- end to end through the public API from pinned host buffers (e2e) ----
     # fresh batches (other embeddings AND other identities' rows than the ones just enqueued: a re-fed embedding makes its target
@@ -548,7 +563,12 @@ def main():
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--no-aux', action='store_true', help='skip the per-kernel HBM micro timings')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the loss and embedding gradients of the last timed step to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes what our kernels computed: --impl ours only')
     w = WORKLOADS[args.workload]
     if args.impl == 'reference':
         run_reference(args, w)

@@ -67,6 +67,26 @@ def test_reference_arm_json_line():
     assert r.returncode == 0 and r.stdout.strip() == ''
 
 
+def test_dump_outputs_files(tmp_path):
+    """--dump-outputs: one float32 .npy per returned array (loss, dLoss/dx, dLoss/dy), a rank suffix when sharded"""
+    import numpy as np
+    b = _bench()
+    out = (torch.tensor(3.25), torch.randn(6, 4), torch.randn(6, 4, dtype=torch.float64))
+    b.dump_outputs(str(tmp_path / 'one'), out, 0, 1)
+    assert sorted(os.listdir(tmp_path / 'one')) == ['dx.npy', 'dy.npy', 'loss.npy']
+    for name, t in zip(('loss', 'dx', 'dy'), out):
+        a = np.load(tmp_path / 'one' / f'{name}.npy')
+        assert a.dtype == np.float32 and a.shape == tuple(t.shape) and np.array_equal(a, t.float().numpy())
+    b.dump_outputs(str(tmp_path / 'sharded'), out, 3, 4)
+    assert sorted(os.listdir(tmp_path / 'sharded')) == ['dx_rank3.npy', 'dy_rank3.npy', 'loss_rank3.npy']
+
+
+def test_steps_and_dump_arguments_are_checked():
+    for extra in (['--steps', '0'], ['--warmup', '-1'], ['--impl', 'reference', '--dump-outputs', 'x']):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py')] + extra, capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and r.stdout == '', (extra, r.stderr)
+
+
 def test_executed_flop_accounting_and_limiter_note():
     """roofline.achieved counts executed tensor FLOPs: every row's cosines, and the gradient sum only for the row tiles that hold a row with a
     softmax term (hard-negative-only rows are swept last and skip GEMM-2); the limiter note counts the W tiles both CTAs of a pair stream."""

@@ -90,19 +90,25 @@ def test_train_one_epoch_sequence(tmp_path):
     assert set(ck) == {'state_dict', 'lru', 'fc', 'qp'}
 
 
-def test_ir100_is_registered_for_c4():
-    """C4 names ResNet-100: the reference defines iresnet100 (resnet_arcface.py:177) but its create_net does not list it"""
+def test_ir100_is_registered_for_c4(tmp_path, monkeypatch):
+    """C4 names ResNet-100: the reference defines iresnet100 (resnet_arcface.py:177) but its create_net does not list it, so create_net
+    takes it from model.resnet_arcface.  Checked against a stand-in `model` package with the reference's layout; without any backbone
+    package on sys.path the name is a ValueError."""
     import sys
     import pytest
     from ffc_b200 import ffc as F_
-    ref = os.environ.get('FFC_REFERENCE_ROOT', '/root/reference')
-    if not os.path.isdir(os.path.join(ref, 'model')):
-        with pytest.raises(ValueError):
-            F_.create_net('ir100', feat_dim=512)
-        return
-    sys.path.insert(0, ref)
+    for name in ('model', 'model.resnet_arcface'):
+        monkeypatch.delitem(sys.modules, name, raising=False)
+    with pytest.raises(ValueError):
+        F_.create_net('ir100', feat_dim=512)
+    pkg = tmp_path / 'model'
+    pkg.mkdir()
+    (pkg / '__init__.py').write_text('def create_net(net_type, **kwargs):\n    return ("create_net", net_type, kwargs)\n')
+    (pkg / 'resnet_arcface.py').write_text('def iresnet100(**kwargs):\n    return ("iresnet100", kwargs)\n')
+    monkeypatch.syspath_prepend(str(tmp_path))
     try:
-        net = F_.create_net('ir100', feat_dim=512, fp16=False)
-        assert sum(p.numel() for p in net.parameters()) > 60e6            # 65.2 M (SURVEY 8(f))
+        assert F_.create_net('ir100', feat_dim=512, fp16=False) == ('iresnet100', {'feat_dim': 512, 'fp16': False})
+        assert F_.create_net('ir50', feat_dim=512) == ('create_net', 'ir50', {'feat_dim': 512})      # the others: the package's create_net
     finally:
-        sys.path.remove(ref)
+        for name in ('model', 'model.resnet_arcface'):
+            sys.modules.pop(name, None)
