@@ -351,6 +351,29 @@ int ffc_head_finalize_gathered_ex(ffc_head_t* h, const ffc_head_pass* in, const 
 int ffc_head_set_dqueue(ffc_head_t* h, int enable);
 int ffc_head_dqueue(ffc_head_t* h, const ffc_head_pass* in, float* dqueue_out, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * 1:N identification against the resident prototypes (nothing like it in the reference: its test
+ * chapter is empty).  The gallery of handle `h` is row queue[0][s] of every slot s < cur_idx of `lru`
+ * (the LRU whose slots index this handle's queue; [0, cur_idx) is exactly the occupied set).  For each
+ * query row: the k prototypes of highest cosine, ordered by score descending, ties by smaller slot.
+ * score_out [n, k] fp32: fp64-accumulated dot of the query row with the fp32 queue row (x_f32 rows are
+ * expected L2-normalised); label_out [n, k] int64: the slot's key; slot_out [n, k] int32: GLOBAL slot
+ * (col_offset + local slot).  Fewer than k resident: the missing entries are slot -1, label INT64_MIN,
+ * score -inf.  bf16 handles select the candidates by the tcgen05 bf16 cosine and rescore them; check-mode
+ * handles (FFC_PREC_FP32) select by the fp32 score itself.  Reads the LRU's device state (cur_idx,
+ * slot keys) without touching recency, and writes nothing but the outputs and the workspace.  No host sync;
+ * two kernel launches per call (bf16: plus one memset), whatever n and cur_idx are.  1 <= k <= FFC_TOPK_MAX,
+ * 1 <= n <= FFC_IDENTIFY_MAX_ROWS (callers split larger inputs).
+ * ---------------------------------------------------------------------------------------------- */
+#define FFC_IDENTIFY_MAX_ROWS 65536
+int ffc_identify_workspace_bytes(ffc_head_t* h, int n, int k, int64_t* bytes_out);
+/* x_f32: [n, D] unit rows.  Searches this handle's q_local slots [0, cur_idx of `lru`); slot_out holds GLOBAL slots.
+ * queue_f32 / queue_bf16: [2, q_local, D] as for a head pass (queue_bf16 may be NULL in check mode); workspace: device memory of
+ * ffc_identify_workspace_bytes bytes, 256-byte aligned, not shared with a call that may run concurrently. */
+int ffc_identify(ffc_head_t* h, const ffc_lru_t* lru, const float* x_f32, int n, int k, const float* queue_f32,
+                 const void* queue_bf16, void* workspace, int64_t workspace_bytes,
+                 float* score_out, int64_t* label_out, int32_t* slot_out, void* stream);
+
 /* sizes in bytes of the five stats arrays for n rows (one rank's worth) */
 int ffc_head_stats_bytes(const ffc_head_config* cfg, int n_rows, int64_t sizes_out[5]);
 

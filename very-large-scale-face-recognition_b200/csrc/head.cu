@@ -13,7 +13,7 @@
 #include <math.h>
 #include <vector>
 
-#include "head_internal.cuh"
+#include "identify_internal.cuh"
 
 namespace ffc {
 struct ReduceJobs;
@@ -1796,4 +1796,50 @@ extern "C" int ffc_head_dqueue(ffc_head_t* h, const ffc_head_pass* in, float* dq
   dq_hard_neg_kernel<<<n, 128, 0, s>>>(h->p16, h->is_out, h->coef, h->nslot, h->wslot, h->wrow, n, D, c.q_local, c.col_offset, dqueue_out);
   FFC_LAUNCH_CHECK();
   return FFC_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// 1:N identification against queue[0] (identify_sm100.cu)
+// ------------------------------------------------------------------------------------------------
+extern "C" int ffc_identify_workspace_bytes(ffc_head_t* h, int n, int k, int64_t* bytes_out) {
+  FFC_REQUIRE(n >= 1 && n <= FFC_IDENTIFY_MAX_ROWS, "ffc_identify_workspace_bytes: n=%d rows outside [1, %d]", n, FFC_IDENTIFY_MAX_ROWS);
+  FFC_REQUIRE(k >= 1 && k <= KMAX, "ffc_identify_workspace_bytes: k=%d outside [1, %d]", k, KMAX);
+  FFC_REQUIRE(h && bytes_out, "ffc_identify_workspace_bytes: NULL argument");
+  *bytes_out = identify_workspace_bytes(h->cfg.precision == FFC_PREC_BF16, n, k, h->cfg.q_local);
+  return FFC_OK;
+}
+
+extern "C" int ffc_identify(ffc_head_t* h, const ffc_lru_t* lru, const float* x_f32, int n, int k, const float* queue_f32, const void* queue_bf16,
+                            void* workspace, int64_t workspace_bytes, float* score_out, int64_t* label_out, int32_t* slot_out, void* stream) {
+  FFC_REQUIRE(n >= 1 && n <= FFC_IDENTIFY_MAX_ROWS, "ffc_identify: n=%d rows outside [1, %d] (split larger inputs)", n, FFC_IDENTIFY_MAX_ROWS);
+  FFC_REQUIRE(k >= 1 && k <= KMAX, "ffc_identify: k=%d outside [1, %d]", k, KMAX);
+  FFC_REQUIRE(h && lru, "ffc_identify: NULL head or LRU handle");
+  FFC_REQUIRE(x_f32 && queue_f32 && workspace && score_out && label_out && slot_out, "ffc_identify: NULL device pointer");
+  const ffc_head_config& c = h->cfg;
+  const bool bf16 = c.precision == FFC_PREC_BF16;
+  FFC_REQUIRE(!bf16 || queue_bf16, "ffc_identify: the bf16 path needs the bf16 queue mirror");
+  const int64_t need = identify_workspace_bytes(bf16, n, k, c.q_local);
+  FFC_REQUIRE(workspace_bytes >= need, "ffc_identify: workspace of %lld bytes, %lld needed", (long long)workspace_bytes, (long long)need);
+  const int32_t* cur_idx = nullptr;
+  const int64_t* slot_key = nullptr;
+  int64_t cap = 0;
+  int rc = lru_device_state(lru, &cur_idx, &slot_key, &cap);
+  if (rc) return rc;
+  FFC_REQUIRE(cap <= c.q_local, "ffc_identify: LRU capacity %lld exceeds the head's %lld queue slots", (long long)cap, (long long)c.q_local);
+  IdentifyArgs a;
+  a.x = x_f32;
+  a.queue_f32 = queue_f32;
+  a.queue_bf16 = bf16 ? queue_bf16 : nullptr;
+  a.q_local = c.q_local;
+  a.col_offset = c.col_offset;
+  a.cur_idx_dev = cur_idx;
+  a.slot_key = slot_key;
+  a.n_rows = n;
+  a.D = c.feat_dim;
+  a.k = k;
+  a.workspace = workspace;
+  a.score_out = score_out;
+  a.label_out = label_out;
+  a.slot_out = slot_out;
+  return launch_identify(h->sm100, a, (cudaStream_t)stream);
 }

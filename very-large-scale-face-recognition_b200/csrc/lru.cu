@@ -26,6 +26,7 @@
 #include <cub/block/block_scan.cuh>
 
 #include "ffc_common.cuh"
+#include "identify_internal.cuh"
 
 namespace ffc {
 
@@ -1052,6 +1053,16 @@ extern "C" int ffc_lru_undo(ffc_lru_t* h, int64_t steps, uint8_t* qpos_dev, void
   h->ht_used_ub += m;    // re-inserted old keys may consume never-used cells
   return FFC_OK;
 }
+
+namespace ffc {
+int lru_device_state(const ffc_lru_t* h, const int32_t** cur_idx_dev, const int64_t** slot_key, int64_t* capacity) {
+  FFC_REQUIRE(h != nullptr, "NULL LRU handle");
+  *cur_idx_dev = &h->st->cur_idx;
+  *slot_key = h->slot_key;
+  *capacity = h->cap;
+  return FFC_OK;
+}
+}  // namespace ffc
 
 extern "C" int ffc_lru_size(ffc_lru_t* h, int64_t* cur_idx_out, int64_t* journal_len_out, void* stream) {
   FFC_REQUIRE(h != nullptr, "ffc_lru_size: NULL handle");

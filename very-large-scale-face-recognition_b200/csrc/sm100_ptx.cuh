@@ -184,6 +184,7 @@ __device__ __forceinline__ uint32_t max_bf16x2(uint32_t a, uint32_t b) {
 // the chunk (5 bits: up to 32 columns; value error 2^-18).  tk[] descending keys (0 = empty), tc[] first column of the chunk a key came from.
 // Warp-collective: all lanes run the same code; a lane with a candidate (key above its threshold `kth`) extracts its largest
 // remaining key per round until no lane has any left.  `kfloor` is the row's threshold shared by the column chunks (below).
+// SIGNED (identification, cosines of any sign): the keys are topk_ord() of the cosine bits instead, and INT_MIN means empty.
 // sorted insertion of one key into the branch-free register list (the caller has checked xk > kth)
 __device__ __forceinline__ void topk_insert_key(int xk, int xc, int k, int (&tk)[KMAX], int (&tc)[KMAX]) {
 #pragma unroll
@@ -199,20 +200,24 @@ __device__ __forceinline__ void topk_insert_key(int xk, int xc, int k, int (&tk)
   }
 }
 
-template <int BASE, int NV>
+// order-preserving map of float bits to int32 (any sign): x < y  <=>  topk_ord(x) < topk_ord(y)
+__host__ __device__ __forceinline__ int topk_ord(uint32_t bits) { return (int)bits >= 0 ? (int)bits : (int)(bits ^ 0x7fffffffu); }
+
+template <int BASE, int NV, bool SIGNED = false>
 __device__ __forceinline__ void topk_scan16(const uint32_t (&v)[NV], uint32_t excl, int col0, bool outl, int k, int (&tk)[KMAX], int (&tc)[KMAX],
                                             int& kth, int kfloor) {
+  constexpr int EMPTY = SIGNED ? (int)0x80000000u : 0;
   int key[16];
 #pragma unroll
   for (int c = 0; c < 16; ++c) {
-    key[c] = (int)((v[BASE + c] & TOPK_VAL_MASK) | (uint32_t)c);
-    if ((excl >> c) & 1u) key[c] = 0;
+    key[c] = (int)(((SIGNED ? (uint32_t)topk_ord(v[BASE + c]) : v[BASE + c]) & TOPK_VAL_MASK) | (uint32_t)c);
+    if ((excl >> c) & 1u) key[c] = EMPTY;
   }
   int bound = 0x7fffffff;      // keys >= bound were already extracted in this chunk
   while (true) {
-    int mx = 0;
+    int mx = EMPTY;
 #pragma unroll
-    for (int c = 0; c < 16; ++c) mx = max(mx, key[c] < bound ? key[c] : 0);
+    for (int c = 0; c < 16; ++c) mx = max(mx, key[c] < bound ? key[c] : EMPTY);
     const bool has = outl && mx > kth;
     if (!__any_sync(0xffffffffu, has)) break;
     if (has) {
@@ -233,7 +238,7 @@ __device__ __forceinline__ void topk_scan16(const uint32_t (&v)[NV], uint32_t ex
         if (r == k - 1) kth = max(tk[r], kfloor);     // own k-th, or the row's shared threshold if that is higher
       bound = mx;
     } else {
-      bound = 0;               // this lane is done with the chunk
+      bound = EMPTY;           // this lane is done with the chunk
     }
   }
 }

@@ -12,6 +12,7 @@ PRECISIONS = {'bf16': 0, 'fp32': 1}
 LRU_MAX_BATCH = 1024     # keys per chunk of the resolve CTA
 LRU_MAX_KEYS = 65536     # keys per ffc_lru_assign call
 TOPK_MAX = 10
+IDENTIFY_MAX_ROWS = 65536  # query rows per ffc_identify call
 KEY_RESERVED = (-(1 << 63), -(1 << 63) + 1)
 
 c_void_p, c_int, c_int32, c_int64, c_float = C.c_void_p, C.c_int, C.c_int32, C.c_int64, C.c_float
@@ -93,6 +94,8 @@ PROTOTYPES = {
     'ffc_head_set_timing': (c_int, [c_void_p, c_int]),
     'ffc_head_get_timing': (c_int, [c_void_p, C.POINTER(C.c_double), C.POINTER(c_int64)]),
     'ffc_head_stats_bytes': (c_int, [C.POINTER(HeadConfig), c_int, C.POINTER(c_int64)]),
+    'ffc_identify_workspace_bytes': (c_int, [c_void_p, c_int, c_int, C.POINTER(c_int64)]),
+    'ffc_identify': (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
 }
 
 _lib = None

@@ -29,6 +29,7 @@ import torch.distributed as dist
 
 from . import _capi
 from ._capi import HeadConfig, HeadPass, HeadStats, check
+from . import identify as _ident
 from .ffc import hard_neg_k
 from .lru import LRU
 
@@ -105,6 +106,12 @@ class CudaShardBackend:
         return dict(red=red, osum=torch.empty(4, n, D, dtype=torch.float32, device=dev),
                     topv=torch.empty(n_ranks, 3, n, k, dtype=torch.float32, device=dev),
                     topi=torch.empty(n_ranks, 3, n, k, dtype=torch.int32, device=dev))
+
+    def identify_local(self, x, k):
+        """Top-k of the rows `x` [n, D] (L2-normalised here) over this shard's resident slots: global slots, labels from this
+        rank's LRU (FFCHead.identify's semantics)."""
+        xn = _ident.normalized_queries(x, self.D, self.dev)
+        return _ident.search(self.lib, self._h, self.lru._h, xn, k, self.queue, self.queue_bf16 if self._cfg.precision == _capi.PRECISIONS['bf16'] else None)
 
     # -- pass steps -------------------------------------------------------------------------------
     def assign(self, keys_compact, n_dev, journal):
@@ -846,6 +853,38 @@ class ShardedFFCHead:
     def forward(self, x, y, x_label, y_label):
         """ffc.py:264-267 with embeddings in (rollback pass, then commit pass)."""
         return self.head(x, y.detach(), x_label, y_label, commit=False) + self.head(y, x.detach(), y_label, x_label, commit=True)
+
+    def identify(self, x, k=1):
+        """1:N identification across the shards (collective: every rank calls it with its own rows, any number of them).  The
+        queries are all-gathered, every rank searches its shard (its LRU's resident slots) with :meth:`FFCHead.identify`'s
+        semantics, one all-gather exchanges the packed candidates, and each rank merges its own rows by (score desc, slot asc):
+        the result equals a one-GPU search over the union of the shards.  Returns ``Identification`` [N, k] for this rank's rows."""
+        k = _ident.check_k(k)
+        be, R, dev = self.backend, self.R, self.dev
+        with torch.no_grad():
+            if self._side is not None:
+                torch.cuda.current_stream(dev).wait_stream(self._side)    # bookkeeping already enqueued (a prefetch undoes itself)
+            x = torch.as_tensor(x)
+            n = x.shape[0] if x.dim() >= 1 else 0
+            counts = self._all_gather(torch.tensor([n], dtype=torch.int64, device=dev)).tolist()
+            n_max = max(counts)
+            if n_max == 0:
+                return _ident.empty(0, k, dev)
+            if n and (x.dim() != 2 or x.shape[1] != self.D):
+                raise ValueError(f'identify expects [N, {self.D}] embeddings, got {tuple(x.shape)}')
+            pad = torch.zeros(n_max, self.D, dtype=getattr(be, 'dtype', torch.float32), device=dev)
+            pad[:n] = x.to(device=dev, dtype=pad.dtype)
+            x_all = self._all_gather(pad)                                    # [R * n_max, D] raw rows (zero rows pad)
+            loc = be.identify_local(x_all, k)
+            # one all-gather of (score, label, slot) packed as 3 x 8-byte words per entry
+            pack = torch.stack([loc.scores.double().view(torch.int64), loc.labels, loc.slots.long()], dim=-1)     # [R * n_max, k, 3]
+            allp = self._all_gather(pack).view(R, R, n_max, k, 3)[:, self.rank, :n]     # [source rank, own rows, k, 3]
+            cand = allp.permute(1, 0, 2, 3).reshape(n, R * k, 3)
+            out = _ident.merge(cand[..., 0].contiguous().view(torch.float64).float(), cand[..., 1], cand[..., 2].to(torch.int32), k)
+            if self._side is not None:
+                self._lru_main_ev = torch.cuda.Event()
+                self._lru_main_ev.record()                                   # a later prefetch must not rewrite the LRU under the search
+        return out
 
     def barrier_timeouts(self):
         """Number of in-kernel cross-rank barriers (gradient slabs, record exchange) that gave up waiting for a peer (5 s) since

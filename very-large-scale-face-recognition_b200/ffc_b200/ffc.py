@@ -17,6 +17,7 @@ import torch
 from torch.nn import Module
 
 from . import _capi
+from . import identify as _ident
 from ._capi import HeadConfig, HeadPass, HeadStats, check
 from .lru import LRU
 from .tail import l2_normalize
@@ -404,6 +405,28 @@ class FFCHead(Module):
         """One head pass: ``forward_impl`` (commit=True, ffc.py:153-204) or ``forward_impl_rollback`` (commit=False,
         ffc.py:208-260) with embeddings in.  Returns the loss; gradients flow to ``p`` only."""
         return _HeadFn.apply(p, self, g, probe_label, gallery_label, commit)
+
+    @torch.no_grad()
+    def identify(self, x, k=1):
+        """1:N identification of embeddings ``x`` [N, D] (fp32 / fp16 / bf16, any device; raw features or unit rows: they are
+        L2-normalised here) against the resident prototypes ``queue[0][s]``, ``s < lru.cur_idx``.  Returns
+        ``Identification(scores, labels, slots)``, device tensors [N, k]: cosine (fp32), the identity's label, its slot; ordered by
+        score descending, ties by smaller slot; fewer than k resident -> slot -1, label INT64_MIN, score -inf.  ``precision='fp32'``
+        heads select by the fp32 score (the check mode), bf16 heads by the tcgen05 bf16 cosine and rescore the k winners in fp32.
+        Leaves queue, mirror, LRU (contents and recency), queue positions and a pending :meth:`prefetch_labels` untouched."""
+        k = _ident.check_k(k)
+        self._ensure()
+        with torch.cuda.device(self._dev):
+            main = torch.cuda.current_stream(self._dev)
+            ev = torch.cuda.Event()
+            ev.record(self._side)              # the bookkeeping enqueued so far (a prefetch's rollback has undone itself by then)
+            main.wait_event(ev)
+            xn = _ident.normalized_queries(x, self.feat_dim, self._dev)
+            if xn.shape[0] == 0:
+                return _ident.empty(0, k, self._dev)
+            out = _ident.search(self._lib, self._h, self._lru._h, xn, k, self.queue, self.queue_bf16 if self.precision == 'bf16' else None)
+            self._lru_sync_main = True         # the next bookkeeping must not rewrite the LRU while the search reads it
+        return out
 
     def last_bookkeeping(self):
         """(rows, cols, labels, ones) of the most recent pass as Python lists (debug / parity tests; synchronises)."""
