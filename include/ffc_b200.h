@@ -343,11 +343,15 @@ int ffc_head_finalize_gathered_ex(ffc_head_t* h, const ffc_head_pass* in, const 
 
 /* Optional mode, off by default: dLoss/dQueue.  The reference keeps `queue` a no-grad buffer (ffc.py:29); a caller that trains the
  * prototypes enables the mode before a pass (ffc_head_set_dqueue: the fused finalize then also exports its per-row coefficients)
- * and, after ffc_head_pass_single / ffc_head_finalize_gathered[_ex] of that pass and before the queue rows change again, calls
- * ffc_head_dqueue: dqueue_out [2, q_local, D] fp32 is OVERWRITTEN with d(loss of the pass)/d(queue) for an upstream gradient of 1 --
- * both add_margin terms (ffc.py:195-202 through autograd, had `queue` required grad) incl. the hard-negative rows.  One more sweep
- * of the tcgen05 kernel with the roles of queue and probe rows swapped (4 n Q D FLOPs, no B x Q matrix) plus two small kernels for
- * the target / `ones` rows and the hard negatives.  bf16 AM / Arc only.  `in` = the pass just finalized. */
+ * and, after the finalize of that pass (ffc_head_pass_single, ffc_head_finalize or ffc_head_finalize_gathered[_ex]) and before the
+ * queue rows change again, calls ffc_head_dqueue: dqueue_out [2, q_local, D] fp32 is OVERWRITTEN with d(loss of the pass)/d(queue)
+ * for an upstream gradient of 1 -- both add_margin terms (ffc.py:195-202 through autograd, had `queue` required grad) incl. the
+ * hard-negative rows.  Every loss type (SV: the hard mask is not differentiated, its 1.2 z + 0.2 transform is) and both precisions.
+ * bf16: one more sweep of the tcgen05 kernel with the roles of queue and probe rows swapped (4 n Q D FLOPs, no B x Q matrix) plus two
+ * small kernels for the target / `ones` rows and the hard negatives; needs `in->queue_bf16`.  Check mode (FFC_PREC_FP32): SIMT
+ * kernels with fp64 accumulation in a fixed order, bit-identical from run to run; needs `in->p_f32` and `in->queue_f32`.  On a shard
+ * the result covers the handle's q_local slots: rows [col_offset, col_offset + q_local) of the gradient of the global queue, since
+ * every rank sweeps all gathered probe rows and finalize's per-row coefficients are global.  `in` = the pass just finalized. */
 int ffc_head_set_dqueue(ffc_head_t* h, int enable);
 int ffc_head_dqueue(ffc_head_t* h, const ffc_head_pass* in, float* dqueue_out, void* stream);
 

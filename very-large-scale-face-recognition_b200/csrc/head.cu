@@ -51,7 +51,8 @@ struct ffc_head {
   ffc::Sm100Cache* sm100;
   // queue-gradient mode (ffc_head_set_dqueue / ffc_head_dqueue)
   int want_dq;
-  __nv_bfloat16* pc16;         // [max_rows][D] probe rows scaled by their softmax coefficients (GEMM-2 operand of the swapped sweep)
+  __nv_bfloat16* pc16;         // [max_rows][D] probe rows scaled by their softmax coefficients (GEMM-2 operand of the swapped sweep; bf16 AM / Arc)
+  float4* dq_col;              // [max_rows] (thr_1, thr_2, a_1, a_2) per probe row: the column scalars of the swapped SV sweep (bf16 SV)
   float* dq_l;                 // [q_local] scratch partials of the swapped sweep (denominators: unused)
   float* dq_tv;                // [q_local]
   int32_t* dq_ti;              // [q_local]
@@ -1177,6 +1178,7 @@ extern "C" int ffc_head_destroy(ffc_head_t* h) {
   cudaFree(h->part_ctr);
   cudaFree(h->kth_shared);
   cudaFree(h->pc16);
+  cudaFree(h->dq_col);
   cudaFree(h->dq_l);
   cudaFree(h->dq_tv);
   cudaFree(h->dq_ti);
@@ -1642,6 +1644,11 @@ extern "C" int ffc_head_get_timing(ffc_head_t* h, double* total_ms_out, int64_t*
 // so dqueue[0] comes out of TMEM row tile by row tile: 4 n Q D more FLOPs per pass, no B x Q matrix.  The <= 2n "special" slots --
 // targets T (the margin changes their coefficient) and `ones` C (losses 1 / 2 read different rows) -- are recomputed exactly by a
 // small SIMT kernel and overwritten; the hard-negative term adds w_neg p_i to the <= 2k rows each outlier row selected.
+// SV: the hardness test cos_ij > thr_l,i is per probe row, i.e. per COLUMN of the swapped sweep, and the two losses' p~ differ where
+// their thresholds do.  The sweep's DQ_SV mode forms the combined weight sum_l a_l,i p~_l,ij h'_l,ij (h' = 1.2 on hard columns, else
+// 1; z = 1.2 cos + 0.2 there) in its epilogue from per-column scalars and accumulates the raw probe rows.
+// Check mode (FFC_PREC_FP32): one SIMT kernel per queue slot with fp64 dots and sums in a fixed order computes every row -- bulk,
+// targets and `ones` alike -- and a one-owner-per-feature kernel adds the hard negatives: no atomics, bit-identical from run to run.
 // ------------------------------------------------------------------------------------------------
 namespace ffc {
 
@@ -1652,13 +1659,31 @@ __global__ void __launch_bounds__(128) dq_scale_probe_kernel(const __nv_bfloat16
   for (int d = threadIdx.x; d < D; d += blockDim.x) pc16[(int64_t)i * D + d] = __float2bfloat16(c * __bfloat162float(p16[(int64_t)i * D + d]));
 }
 
+// per probe row: (thr_1, thr_2, a_1, a_2), the coefficients zero on hard-negative-only rows (their term is dq_hard_neg_kernel's)
+__global__ void __launch_bounds__(128) dq_sv_cols_kernel(const float* __restrict__ thr, const float* __restrict__ coef, const uint8_t* __restrict__ is_out, int n,
+                                                         float4* __restrict__ col) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const bool o = is_out[i];
+  col[i] = make_float4(thr[i], thr[n + i], o ? 0.f : coef[0 * n + i], o ? 0.f : coef[1 * n + i]);
+}
+
+// p~ h' of one non-target cosine: SV (thr != NULL) applies the hard-example transform above the row's threshold
+__device__ __forceinline__ float dq_pt(float dot, float a2, float b2, float th) {
+  const bool m = dot > th;
+  return exp2f(fmaf(m ? fmaf(SV_T, dot, SV_T - 1.f) : dot, a2, -b2)) * (m ? SV_T : 1.f);
+}
+
 // one block per candidate special slot: blocks [0, max_rows) take ones_list[b] (if b < n_ones), blocks [max_rows, max_rows + n) the
-// target of probe row b - max_rows (if it is local, not in C -- those are the first kind -- and not claimed by another row's block)
+// target of probe row b - max_rows (if it is local, not in C -- those are the first kind -- and not claimed by another row's block).
+// SV: `thr` [2][n] holds the per-row thresholds of the two losses.
+template <bool SV>
 __global__ void __launch_bounds__(256) dq_special_rows_kernel(const __nv_bfloat16* __restrict__ p16, const __nv_bfloat16* __restrict__ qh, int64_t q_local, int D, int n,
                                                               int max_rows, const int32_t* __restrict__ ones_list, const int32_t* __restrict__ n_ones_p,
                                                               const uint32_t* __restrict__ cmask_unused, const int32_t* __restrict__ tcol,
                                                               const int32_t* __restrict__ tpos, const uint8_t* __restrict__ is_out, const float* __restrict__ coef,
-                                                              float a2, float b2, int32_t* __restrict__ claim, int32_t epoch, float* __restrict__ dq) {
+                                                              const float* __restrict__ thr, float a2, float b2, int32_t* __restrict__ claim, int32_t epoch,
+                                                              float* __restrict__ dq) {
   extern __shared__ float sm[];          // [D] queue row, [n] coefficients
   float* s_q = sm;
   float* s_c = sm + D;
@@ -1700,8 +1725,13 @@ __global__ void __launch_bounds__(256) dq_special_rows_kernel(const __nv_bfloat1
             dot = fmaf(v.x, s_q[d], dot);
             dot = fmaf(v.y, s_q[d + 1], dot);
           }
-          const float pt = exp2f(fmaf(dot, a2, -b2));
-          c = in_c ? coef[r * n + i] * pt : (coef[0 * n + i] + coef[1 * n + i]) * pt;
+          if (SV) {
+            c = in_c ? coef[r * n + i] * dq_pt(dot, a2, b2, thr[r * n + i])
+                     : coef[0 * n + i] * dq_pt(dot, a2, b2, thr[i]) + coef[1 * n + i] * dq_pt(dot, a2, b2, thr[n + i]);
+          } else {
+            const float pt = exp2f(fmaf(dot, a2, -b2));
+            c = in_c ? coef[r * n + i] * pt : (coef[0 * n + i] + coef[1 * n + i]) * pt;
+          }
         }
       }
       s_c[i] = c;
@@ -1731,14 +1761,92 @@ __global__ void __launch_bounds__(128) dq_hard_neg_kernel(const __nv_bfloat16* _
   }
 }
 
+// Check mode: one block per local slot j writes dqueue[0][j] and dqueue[1][j] whole.  Per probe row i (fp64 on the fp32 inputs):
+//   target of i (tcol[i] == j):  d/dcos of the margined logit from finalize (cT), loss 2's on queue[1] iff j is in C
+//   otherwise:                   a_l,i p~_l,ij h'_l,ij, with loss 2 reading queue[1][j] iff j is in C (and nothing reading it else)
+// hard-negative-only rows contribute nothing here (dq_hard_neg_f32_kernel).  Sums over i run in index order.
+__global__ void __launch_bounds__(128) dq_rows_f32_kernel(const float* __restrict__ P, const float* __restrict__ qf, int64_t q_local, int D, int n,
+                                                          const uint32_t* __restrict__ cmask, const int32_t* __restrict__ tcol, const uint8_t* __restrict__ is_out,
+                                                          const float* __restrict__ coef, const float* __restrict__ thr, double s, double M,
+                                                          float* __restrict__ dq) {
+  extern __shared__ double smd[];        // [2][D] queue rows, [2][n] coefficients
+  double* s_q = smd;
+  double* s_c = smd + 2 * D;
+  const int64_t j = blockIdx.x;
+  const bool in_c = cmask && ((cmask[j >> 5] >> (j & 31)) & 1u);
+  for (int d = threadIdx.x; d < D; d += blockDim.x) {
+    s_q[d] = qf[j * D + d];
+    s_q[D + d] = qf[(q_local + j) * D + d];
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    double c0 = 0.0, c1 = 0.0;      // coefficients of p_i in dqueue[0][j] and dqueue[1][j]
+    if (!is_out[i]) {
+      if (tcol[i] == j) {
+        c0 = coef[2 * n + i];
+        if (in_c) c1 = coef[3 * n + i]; else c0 += coef[3 * n + i];
+      } else {
+        const float* pr = P + (int64_t)i * D;
+        double dot[2] = {0.0, 0.0};
+        for (int d = 0; d < D; ++d) dot[0] += (double)pr[d] * s_q[d];
+        if (in_c)
+          for (int d = 0; d < D; ++d) dot[1] += (double)pr[d] * s_q[D + d];
+        else
+          dot[1] = dot[0];
+        double g[2];
+        for (int l = 0; l < 2; ++l) {
+          const bool hard = thr && dot[l] > (double)thr[l * n + i];
+          const double z = hard ? (double)SV_T * dot[l] + (double)SV_T - 1.0 : dot[l];
+          g[l] = (double)coef[l * n + i] * exp(s * z - M) * (hard ? (double)SV_T : 1.0);
+        }
+        c0 = g[0];
+        if (in_c) c1 = g[1]; else c0 += g[1];
+      }
+    }
+    s_c[i] = c0;
+    s_c[n + i] = c1;
+  }
+  __syncthreads();
+  for (int d = threadIdx.x; d < D; d += blockDim.x) {
+    double a0 = 0.0, a1 = 0.0;
+    for (int i = 0; i < n; ++i) {
+      const double pv = P[(int64_t)i * D + d];
+      a0 += s_c[i] * pv;
+      a1 += s_c[n + i] * pv;
+    }
+    dq[j * D + d] = (float)a0;
+    dq[(q_local + j) * D + d] = (float)a1;
+  }
+}
+
+// Check mode, hard negatives: a thread owns feature d of every destination row and walks the outlier rows and their selections in
+// order -- deterministic where dq_hard_neg_kernel's atomics are not
+__global__ void __launch_bounds__(128) dq_hard_neg_f32_kernel(const float* __restrict__ P, const uint8_t* __restrict__ is_out, const float* __restrict__ coef,
+                                                              const int32_t* __restrict__ nslot, const int32_t* __restrict__ wslot, const uint8_t* __restrict__ wrow,
+                                                              int n, int D, int64_t q_local, int64_t col_offset, float* __restrict__ dq) {
+  const int d = blockIdx.x * blockDim.x + threadIdx.x;
+  if (d >= D) return;
+  for (int i = 0; i < n; ++i) {
+    if (!is_out[i]) continue;
+    const float w = coef[0 * n + i] * P[(int64_t)i * D + d];
+    for (int x = 0; x < nslot[i]; ++x) {
+      const int64_t loc = (int64_t)wslot[(int64_t)i * 2 * KMAX + x] - col_offset;
+      if (loc >= 0 && loc < q_local) dq[((int64_t)wrow[(int64_t)i * 2 * KMAX + x] * q_local + loc) * D + d] += w;
+    }
+  }
+}
+
 }  // namespace ffc
 
 extern "C" int ffc_head_set_dqueue(ffc_head_t* h, int enable) {
   FFC_REQUIRE(h != nullptr, "ffc_head_set_dqueue: NULL handle");
-  FFC_REQUIRE(!enable || (h->cfg.precision == FFC_PREC_BF16 && h->cfg.loss_type != FFC_LOSS_SV), "ffc_head_set_dqueue: the queue-gradient mode is built for the bf16 AM / Arc head");
-  if (enable && !h->pc16) {
+  // (check mode needs no scratch: dq_rows_f32_kernel writes every row)
+  if (enable && h->cfg.precision == FFC_PREC_BF16 && !h->dq_claim) {
     const int64_t R = h->cfg.max_rows, D = h->cfg.feat_dim, Q = h->cfg.q_local;
-    FFC_CUDA(cudaMalloc(&h->pc16, R * D * sizeof(__nv_bfloat16)));
+    if (h->cfg.loss_type == FFC_LOSS_SV)
+      FFC_CUDA(cudaMalloc(&h->dq_col, R * sizeof(float4)));
+    else
+      FFC_CUDA(cudaMalloc(&h->pc16, R * D * sizeof(__nv_bfloat16)));
     FFC_CUDA(cudaMalloc(&h->dq_l, Q * sizeof(float)));
     FFC_CUDA(cudaMalloc(&h->dq_tv, Q * sizeof(float)));
     FFC_CUDA(cudaMalloc(&h->dq_ti, Q * sizeof(int32_t)));
@@ -1749,16 +1857,55 @@ extern "C" int ffc_head_set_dqueue(ffc_head_t* h, int enable) {
   return FFC_OK;
 }
 
+template <bool SV>
+static int launch_dq_special_rows(ffc_head_t* h, const ffc_head_pass* in, const __nv_bfloat16* qh, size_t smem, float* dqueue_out, cudaStream_t s) {
+  static bool attr_set = false;
+  if (!attr_set) {
+    FFC_CUDA(cudaFuncSetAttribute(dq_special_rows_kernel<SV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    attr_set = true;
+  }
+  const ffc_head_config& c = h->cfg;
+  dq_special_rows_kernel<SV><<<c.max_rows + in->n_rows, 256, smem, s>>>(h->p16, qh, c.q_local, c.feat_dim, in->n_rows, c.max_rows, in->ones_list, in->n_ones, in->cmask,
+                                                                        h->tcol, h->tpos, h->is_out, h->coef, SV ? h->thr : nullptr, c.scale * 1.4426950408889634f,
+                                                                        fixed_max_of(c) * 1.4426950408889634f, h->dq_claim, h->dq_epoch, dqueue_out);
+  FFC_LAUNCH_CHECK();
+  return FFC_OK;
+}
+
 extern "C" int ffc_head_dqueue(ffc_head_t* h, const ffc_head_pass* in, float* dqueue_out, void* stream) {
   FFC_REQUIRE(h && in && dqueue_out, "ffc_head_dqueue: NULL argument");
   FFC_REQUIRE(h->want_dq, "ffc_head_dqueue: enable the mode with ffc_head_set_dqueue before the pass");
   const ffc_head_config& c = h->cfg;
   const int n = in->n_rows, D = c.feat_dim;
-  FFC_REQUIRE(n >= 1 && n <= c.max_rows && in->queue_bf16 && in->ones_list && in->n_ones, "ffc_head_dqueue: bad pass description");
+  const bool bf16 = c.precision == FFC_PREC_BF16, sv = c.loss_type == FFC_LOSS_SV;
+  FFC_REQUIRE(n >= 1 && n <= c.max_rows && in->ones_list && in->n_ones, "ffc_head_dqueue: bad pass description");
+  FFC_REQUIRE(bf16 ? in->queue_bf16 != nullptr : (in->p_f32 && in->queue_f32), "ffc_head_dqueue: %s", bf16 ? "the bf16 head needs the bf16 queue mirror"
+                                                                                                           : "check mode needs p_f32 and queue_f32");
   FFC_REQUIRE(c.q_local < ((int64_t)1 << 31) / 2, "ffc_head_dqueue: shard too large");
   cudaStream_t s = (cudaStream_t)stream;
+  if (!bf16) {
+    const size_t smem = (size_t)(2 * D + 2 * n) * sizeof(double);
+    FFC_REQUIRE(smem <= 200 * 1024, "ffc_head_dqueue: %d rows exceed the check-mode kernel's shared memory", n);
+    static bool attr_set = false;
+    if (!attr_set) {
+      FFC_CUDA(cudaFuncSetAttribute(dq_rows_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+      attr_set = true;
+    }
+    dq_rows_f32_kernel<<<(unsigned)c.q_local, 128, smem, s>>>(in->p_f32, in->queue_f32, c.q_local, D, n, in->cmask, h->tcol, h->is_out, h->coef, sv ? h->thr : nullptr,
+                                                              (double)c.scale, (double)fixed_max_of(c), dqueue_out);
+    FFC_LAUNCH_CHECK();
+    dq_hard_neg_f32_kernel<<<(D + 127) / 128, 128, 0, s>>>(in->p_f32, h->is_out, h->coef, h->nslot, h->wslot, h->wrow, n, D, c.q_local, c.col_offset, dqueue_out);
+    FFC_LAUNCH_CHECK();
+    return FFC_OK;
+  }
+  const size_t smem = (size_t)(D + n) * sizeof(float);
+  FFC_REQUIRE(smem <= 200 * 1024, "ffc_head_dqueue: %d rows exceed the special-row kernel's shared memory", n);
   const __nv_bfloat16* qh = (const __nv_bfloat16*)in->queue_bf16;
-  dq_scale_probe_kernel<<<n, 128, 0, s>>>(h->p16, h->coef, h->is_out, n, D, h->pc16);
+  if (sv) {
+    dq_sv_cols_kernel<<<(n + 127) / 128, 128, 0, s>>>(h->thr, h->coef, h->is_out, n, h->dq_col);
+  } else {
+    dq_scale_probe_kernel<<<n, 128, 0, s>>>(h->p16, h->coef, h->is_out, n, D, h->pc16);
+  }
   FFC_LAUNCH_CHECK();
   // the swapped sweep: "probe rows" = the queue rows of queue[0], columns = the n probe embeddings
   SweepArgs a;
@@ -1767,7 +1914,8 @@ extern "C" int ffc_head_dqueue(ffc_head_t* h, const ffc_head_pass* in, float* dq
   a.n_rows = (int)c.q_local;
   a.D = D;
   a.W_bf16 = h->p16;
-  a.W2_bf16 = h->pc16;
+  a.W2_bf16 = sv ? nullptr : h->pc16;       // SV: the coefficients are in the epilogue's weights, GEMM-2 sums the raw probe rows
+  a.dq_col = sv ? h->dq_col : nullptr;
   a.force_pair = 1;
   a.n_cols = n;
   a.kth_shared = h->kth_shared;
@@ -1783,16 +1931,7 @@ extern "C" int ffc_head_dqueue(ffc_head_t* h, const ffc_head_pass* in, float* dq
   if (rc) return rc;
   FFC_CUDA(cudaMemsetAsync(dqueue_out + c.q_local * D, 0, (size_t)c.q_local * D * sizeof(float), s));
   h->dq_epoch += 1;
-  const size_t smem = (size_t)(D + n) * sizeof(float);
-  static bool attr_set = false;
-  if (!attr_set) {
-    FFC_CUDA(cudaFuncSetAttribute(dq_special_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    attr_set = true;
-  }
-  FFC_REQUIRE(smem <= 200 * 1024, "ffc_head_dqueue: %d rows exceed the special-row kernel's shared memory", n);
-  dq_special_rows_kernel<<<c.max_rows + n, 256, smem, s>>>(h->p16, qh, c.q_local, D, n, c.max_rows, in->ones_list, in->n_ones, in->cmask, h->tcol, h->tpos, h->is_out, h->coef,
-                                                           c.scale * 1.4426950408889634f, fixed_max_of(c) * 1.4426950408889634f, h->dq_claim, h->dq_epoch, dqueue_out);
-  FFC_LAUNCH_CHECK();
+  if ((rc = sv ? launch_dq_special_rows<true>(h, in, qh, smem, dqueue_out, s) : launch_dq_special_rows<false>(h, in, qh, smem, dqueue_out, s))) return rc;
   dq_hard_neg_kernel<<<n, 128, 0, s>>>(h->p16, h->is_out, h->coef, h->nslot, h->wslot, h->wrow, n, D, c.q_local, c.col_offset, dqueue_out);
   FFC_LAUNCH_CHECK();
   return FFC_OK;

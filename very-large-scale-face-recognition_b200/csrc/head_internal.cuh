@@ -41,6 +41,7 @@ struct SweepArgs {
   float* o_part;                 // [n_chunks][n_rows][D]
   float* topv_part;              // [n_chunks][n_rows][k]   descending, -inf padded
   int32_t* topi_part;            // [n_chunks][n_rows][k]   LOCAL column indices
+  const float4* dq_col;          // optional: the SV queue-gradient sweep's per-column (thr_1, thr_2, a_1, a_2); selects that kernel mode.  CTA-pair kernel only.
 };
 
 int launch_sweep_simt(const SweepArgs& a, cudaStream_t s);

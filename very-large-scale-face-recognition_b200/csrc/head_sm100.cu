@@ -162,7 +162,10 @@ __device__ __forceinline__ Item decode_item(const Sm100Params& prm, int item_all
   return it;
 }
 
-template <bool SV, int D>
+// DQ_SV: the SV queue-gradient sweep (ffc_head_dqueue on an SV head, roles swapped: the columns are the probe rows).  P~ is then the
+// combined weight sum_l a_l,j p~_l,ij h'_l,ij of both losses, from per-column thresholds and coefficients (Sm100Params::dq_col), and
+// GEMM-2 accumulates the raw probe rows.
+template <bool SV, int D, bool DQ_SV = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1)
     ffc_head_sweep_sm100_kernel(const __grid_constant__ CUtensorMap map_p, const __grid_constant__ CUtensorMap map_w1a,
                                 const __grid_constant__ CUtensorMap map_w2a, const __grid_constant__ CUtensorMap map_w1b,
@@ -511,7 +514,34 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1)
             uint32_t pk[16];
             // (hard-negative-only items: no softmax term -- ffc.py:86-92 takes the top-k of the raw cosines and nothing else from these
             // rows -- so no exponentials, no P~ tile, and the O-CTA sits the item out)
-            if (!all_out) {
+            if constexpr (DQ_SV) {
+              // column col0 + lane's (thr_1, thr_2, a_1, a_2), handed to the 32 rows of the warp column by column (a = 0 past the
+              // last column and on hard-negative-only rows).  The two losses' p~ differ only where their hardness does, so one
+              // exponential per element unless the column's thresholds differ (warp-uniform).
+              const float4 cw = (int64_t)col0 + lane < n_cols ? __ldg(prm.dq_col + col0 + lane) : make_float4(INFINITY, INFINITY, 0.f, 0.f);
+  #pragma unroll
+              for (int c = 0; c < 32; c += 2) {
+                float w[2];
+  #pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                  const float t1 = __shfl_sync(0xffffffffu, cw.x, c + e), t2 = __shfl_sync(0xffffffffu, cw.y, c + e);
+                  const float c1 = __shfl_sync(0xffffffffu, cw.z, c + e), c2 = __shfl_sync(0xffffffffu, cw.w, c + e);
+                  const float x = __uint_as_float(v[c + e]);
+                  const bool m1 = x > t1;
+                  const float p1 = ex2f(fmaf(m1 ? fmaf(SV_T, x, SV_T - 1.f) : x, a2, -b2)) * (m1 ? SV_T : 1.f);
+                  if (t1 == t2) {
+                    w[e] = (c1 + c2) * p1;
+                  } else {
+                    const bool m2 = x > t2;
+                    const float p2 = ex2f(fmaf(m2 ? fmaf(SV_T, x, SV_T - 1.f) : x, a2, -b2)) * (m2 ? SV_T : 1.f);
+                    w[e] = fmaf(c1, p1, c2 * p2);
+                  }
+                }
+                l0 += w[0];
+                l1 += w[1];
+                pk[c >> 1] = pack_bf16(w[0], w[1]);
+              }
+            } else if (!all_out) {
   #pragma unroll
               for (int c = 0; c < 32; c += 2) {
                 if (dbg_noEpi) {
@@ -1075,10 +1105,10 @@ int sm100_pick_chunks(int n_rows, int64_t n_cols, int D, int chunk_cap) {
   return best;
 }
 
-template <bool SV, int D>
+template <bool SV, int D, bool DQ_SV = false>
 static int launch_one(const CUtensorMap* maps, const Sm100Params& p, int n_items, cudaStream_t s) {
   static bool attr_set = false;
-  auto kern = ffc_head_sweep_sm100_kernel<SV, D>;
+  auto kern = ffc_head_sweep_sm100_kernel<SV, D, DQ_SV>;
   constexpr size_t smem = SweepShape<D>::SMEM;
   if (!attr_set) {
     FFC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1167,6 +1197,7 @@ int launch_sweeps_sm100(Sm100Cache* cache, const SweepArgs* sweeps, int n_sweeps
   p.a2 = a.scale * LOG2E;
   p.b2 = a.fixed_max * LOG2E;
   p.k = a.k;
+  p.dq_col = a.dq_col;
   p.debug = 0;
 #if FFC_SM100_DEBUG_BUILD
   {
@@ -1223,7 +1254,8 @@ int launch_sweeps_sm100(Sm100Cache* cache, const SweepArgs* sweeps, int n_sweeps
   }
 #define FFC_SWEEP_CASE(DV)                                                       \
   case DV:                                                                       \
-    return a.sv ? launch_one<true, DV>(maps, p, n_items, s) : launch_one<false, DV>(maps, p, n_items, s);
+    return a.dq_col ? launch_one<false, DV, true>(maps, p, n_items, s)                    \
+                    : (a.sv ? launch_one<true, DV>(maps, p, n_items, s) : launch_one<false, DV>(maps, p, n_items, s));
   switch (a.D) {
     FFC_SWEEP_CASE(64)
     FFC_SWEEP_CASE(128)

@@ -279,6 +279,7 @@ struct Sm100Params {
                // 1 = O-CTA skips TMA+MMA, 2 = epilogue skips tcgen05.ld/exp, 4 = S-CTA skips TMA+MMA,
                // 16 = no P~ hand-off (both CTAs free-run), 64 = no W TMA loads (MMAs run on whatever is in shared memory)
   SubSweep sub[MAX_SUB];
+  const float4* dq_col;       // SV queue-gradient sweep only: [n_cols] (thr_1, thr_2, a_1, a_2) per column (= probe row)
 };
 
 // host side (head_sm100.cu): cached tensor maps.  box = 64 features x box_rows rows (K-major, 128-byte swizzle); chunked3d: the same

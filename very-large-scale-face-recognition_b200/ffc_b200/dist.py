@@ -243,6 +243,16 @@ class CudaShardBackend:
         check(self.lib.ffc_head_finalize(self._h, C.byref(hp), C.byref(hs), n_ranks, loss.data_ptr(), dp.data_ptr(), self._s()))
         return loss, dp
 
+    def enable_dqueue(self):
+        """queue-gradient mode of the shard's head (ffc_head_set_dqueue): the finalize kernels also export their per-row coefficients"""
+        check(self.lib.ffc_head_set_dqueue(self._h, 1))
+
+    def dqueue(self, p_all, label, out):
+        """d(loss of the pass just finalized)/d(this shard's queue rows as the pass swept them) into `out` [2, q_local, D] fp32
+        (ffc_head_dqueue): after finalize, before restore_queue()"""
+        hp = self._pass_struct(p_all, label)
+        check(self.lib.ffc_head_dqueue(self._h, C.byref(hp), out.data_ptr(), self._s()))
+
     def end_pass(self):
         self.cmask.zero_()
 
@@ -285,7 +295,7 @@ class ShardedFFCHead:
     """R-way column-sharded head.  ``backend_factory(q_local, col_offset, max_rows) -> backend`` is for the CPU tests."""
 
     def __init__(self, feat_dim, queue_size, scale=32.0, loss_type='AM', margin=0.4, precision='bf16', max_batch=1024, device=None,
-                 group=None, backend_factory=None):
+                 group=None, backend_factory=None, queue_grad=False):
         assert dist.is_initialized(), 'torch.distributed must be initialised (one process per GPU)'
         assert loss_type in ('AM', 'Arc', 'SV')
         self.loss_type = loss_type
@@ -327,11 +337,34 @@ class ShardedFFCHead:
         # reading through the overlay; rollback bookkeeping alternates between sets 0 and 2 so that the next step's (prefetch) never
         # touches the set the current step still needs
         self.merged = bool(getattr(self.backend, 'merged', False)) and not os.environ.get('FFC_DIST_NO_MERGE')
+        # Optional, off by default (FFCHead's queue_grad, per shard): after every pass `dqueue_pass` [2, q_local, D] holds d(loss of that
+        # pass)/d(this rank's queue rows as the pass swept them) -- rows [off, off + q_local) of the gradient of the global queue -- and
+        # `dqueue` accumulates it until zero_dqueue().  It takes the per-pass flow: the merged step finalizes the rollback pass after its
+        # rows have been restored and re-enqueued (reading them through the overlay map), but the swapped sweep reads the queue by TMA.
+        self.queue_grad = bool(queue_grad)
+        self.dqueue = self.dqueue_pass = None
+        if self.queue_grad:
+            self.merged = False
+            self.backend.enable_dqueue()
+            dt = getattr(self.backend, 'dtype', torch.float32)
+            self.dqueue = torch.zeros(2, self.Ql, self.D, dtype=dt, device=self.dev)
+            self.dqueue_pass = torch.zeros(2, self.Ql, self.D, dtype=dt, device=self.dev)
         self._rb_set = 0
         self._set_free = {}         # bookkeeping set -> event: the step that used it last has finished with it
         self._route = None
         if self.merged and self._nccl:
             self._init_route(os.environ.get('FFC_DIST_NO_SYMM') is None)
+
+    def zero_dqueue(self):
+        """Reset the accumulated queue gradient of this rank's shard (queue_grad=True)."""
+        if self.dqueue is not None:
+            self.dqueue.zero_()
+
+    def _dqueue(self, be, p_all, label):
+        if self.queue_grad:      # while the shard still is what the pass swept (a rollback pass restores its rows next)
+            be.dqueue(p_all, label, self.dqueue_pass)
+            self.dqueue.add_(self.dqueue_pass)
+            self._mark('dqueue')
 
     def _init_route(self, try_symm):
         """Staging for the reduce-scatter folded into finalize.  Preferred: a symmetric-memory buffer [R sources][2 passes][B][D] per
@@ -772,6 +805,7 @@ class ShardedFFCHead:
             self._mark('stat_exchange')
             loss, dp_part = be.finalize_gathered(p_all, label, rec, R)
             self._mark('finalize')
+            self._dqueue(be, p_all, label)
             return self._finish_tail(be, dp_part, loss, label, ctx, commit)
         st = self._stats.get(n)
         if st is None:
@@ -804,6 +838,7 @@ class ShardedFFCHead:
         self._mark('stat_exchange')
         loss, dp_part = be.finalize(p_all, label, st, R)
         self._mark('finalize')
+        self._dqueue(be, p_all, label)
         return self._finish_tail(be, dp_part, loss, label, ctx, commit)
 
     def _finish_tail(self, be, dp_part, loss, label, ctx, commit):

@@ -103,7 +103,8 @@ class FFCHead(Module):
         # Optional, off by default (the reference's queue is a no-grad buffer, ffc.py:29): also compute dLoss/dQueue.  After every head
         # pass `dqueue_pass` [2, Q, D] holds d(loss of that pass)/d(queue as the pass swept it) for an upstream gradient of 1, and
         # `dqueue` accumulates it over passes until zero_dqueue() -- a caller that trains the prototypes applies it after
-        # loss.backward(), multiplied by whatever factor scales the loss (a GradScaler's).  bf16 AM / Arc.
+        # loss.backward(), multiplied by whatever factor scales the loss (a GradScaler's).  Every loss type, both precisions (the
+        # check mode's gradient is fp64-accumulated and bit-identical from run to run); ShardedFFCHead has the same option per shard.
         self.queue_grad = bool(queue_grad)
         self.dqueue = self.dqueue_pass = None
         q = torch.rand(2, self.queue_size, self.feat_dim, device=device)                                     # ffc.py:29-30
