@@ -267,7 +267,8 @@ typedef struct ffc_head_pass {
  * noted), n = n_rows, k = topk, D = feat_dim:
  *   lsum   [4][n]      softmax denominators (relative to the fixed max M = c*scale): common under loss 1,
  *                      common under loss 2 (written and read only for SV), side0 (`ones` rows of queue[0]), side1 (queue[1])
- *   osum   [4][n][D]   sum_j p~_ij W_j for the same four column sets
+ *   osum   [4][n][D]   sum_j p~_ij W_j for the same four column sets; zero in the rows of hard-negative-only rows
+ *                      (label -1: no softmax term, finalize never reads them); 16-byte aligned
  *   tgt    [4][n]      cos_t under queue[0], cos_t under W2, (owner flag as 1.0/0.0), spare
  *   topv   [3][n][k]   running top-k cosines (descending; -inf padded), topi int32 [3][n][k] GLOBAL slots
  * On several GPUs the caller sums lsum/tgt across ranks (all-reduce), all-gathers topv/topi, then
@@ -294,13 +295,13 @@ int ffc_head_sweep_prepared(ffc_head_t* h, const ffc_head_pass* in, const ffc_he
  * stats were reduced; dp_out [n_rows, D] fp32 = this rank's contribution to dLoss/dp (the whole
  * gradient on one GPU).  n_ranks_topk: number of gathered top-k candidate sets in stats->topv/topi
  * ([n_ranks][3][n][k]); 1 on one GPU.  n_pos/n_out (global counts of label!=-1 / ==-1 rows) are
- * computed on the device from `label`. */
+ * computed on the device from `label`.  dp_out 16-byte aligned. */
 int ffc_head_finalize(ffc_head_t* h, const ffc_head_pass* in, const ffc_head_stats* stats,
                       int n_ranks_topk, float* loss_out, float* dp_out, void* stream);
 
-/* One-GPU fast path: ffc_head_sweep + ffc_head_finalize(n_ranks_topk = 1) as one call.  On the bf16 AM / Arc path the chunk
- * reduction, the scalar part and dLoss/dp run as ONE kernel after the sweep (the statistics never round-trip through HBM, so
- * `scratch` is left partly unwritten: only tgt is filled); other configurations run the two calls back to back.
+/* One-GPU fast path: ffc_head_sweep + ffc_head_finalize(n_ranks_topk = 1) as one call.  On the bf16 AM / Arc path finalize also
+ * does the chunk reduction of the sweep's partials (the statistics never round-trip through HBM, so `scratch` is left partly
+ * unwritten: only tgt is filled); other configurations run the two calls back to back.
  * Replaces ffc.py:195-202 / 248-254 + loss.backward() of one head pass. */
 int ffc_head_pass_single(ffc_head_t* h, const ffc_head_pass* in, const ffc_head_stats* scratch,
                          float* loss_out, float* dp_out, void* stream);

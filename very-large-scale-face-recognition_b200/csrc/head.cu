@@ -465,48 +465,9 @@ static int simt_pick_chunks(int n_rows, int64_t n_cols) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// reduce partials over chunks -> stats slot `slot` (lsum/osum) and top-k slot `tslot` (or -1)
+// reduce partials over chunks
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) head_reduce_kernel(const float* __restrict__ l_part, const float* __restrict__ o_part,
-                                                          const float* __restrict__ topv_part, const int32_t* __restrict__ topi_part, int n_chunks,
-                                                          int n_rows, int D, int k, float* __restrict__ lsum, float* __restrict__ osum,
-                                                          float* __restrict__ topv, int32_t* __restrict__ topi, const uint8_t* __restrict__ is_out,
-                                                          int64_t idx_base, const int32_t* __restrict__ idx_map) {
-  const int i = blockIdx.x;
-  for (int d = threadIdx.x; d < D; d += blockDim.x) {
-    float acc = 0.f;
-    for (int c = 0; c < n_chunks; ++c) acc += o_part[((int64_t)c * n_rows + i) * D + d];
-    osum[(int64_t)i * D + d] = acc;
-  }
-  if (threadIdx.x == 0) {
-    float acc = 0.f;
-    for (int c = 0; c < n_chunks; ++c) acc += l_part[(int64_t)c * n_rows + i];
-    lsum[i] = acc;
-    if (topv) {
-      float tv[KMAX];
-      int32_t ti[KMAX];
-      for (int q = 0; q < KMAX; ++q) {
-        tv[q] = -INFINITY;
-        ti[q] = -1;
-      }
-      if (is_out[i]) {
-        for (int c = 0; c < n_chunks; ++c)
-          for (int q = 0; q < k; ++q) {
-            const float v = topv_part[((int64_t)c * n_rows + i) * k + q];
-            if (v > tv[k - 1]) topk_insert<KMAX>(tv, ti, k, v, topi_part[((int64_t)c * n_rows + i) * k + q]);
-          }
-      }
-      for (int q = 0; q < k; ++q) {
-        topv[(int64_t)i * k + q] = tv[q];
-        int32_t id = ti[q];
-        if (id >= 0) id = (int32_t)(idx_base + (idx_map ? idx_map[id] : id));   // -> global slot
-        topi[(int64_t)i * k + q] = id;
-      }
-    }
-  }
-}
-
-// The same reduction for up to three sweeps in one launch (blockIdx.y = sweep): the merged main + side launch of the bf16 path.
+// One sweep's chunk partials and where their reduction goes: stats slot lsum / osum, top-k slot topv / topi (NULL: no top-k).
 struct ReduceJob {
   const float* l_part;
   const float* o_part;
@@ -522,12 +483,41 @@ struct ReduceJob {
 };
 struct ReduceJobs {
   ReduceJob j[3];
+  int n;
 };
-__global__ void __launch_bounds__(128) head_reduce_multi_kernel(const ReduceJobs jobs, int n_rows, int D, int k, const uint8_t* __restrict__ is_out) {
+
+// Row i's softmax denominator: the chunk partials summed in chunk order.
+__device__ __forceinline__ float chunk_lsum(const ReduceJob& r, int n_rows, int i) {
+  float acc = 0.f;
+  for (int c = 0; c < r.n_chunks; ++c) acc += r.l_part[(int64_t)c * n_rows + i];
+  return acc;
+}
+
+// Row i's top-k candidates merged over the chunks (only hard-negative-only rows have any), descending and -inf padded, with the
+// winners' columns mapped to global slots (-1: none).
+__device__ __forceinline__ void chunk_topk(const ReduceJob& r, int n_rows, int k, int i, bool outl, float (&tv)[KMAX], int32_t (&ti)[KMAX]) {
+  for (int q = 0; q < KMAX; ++q) {
+    tv[q] = -INFINITY;
+    ti[q] = -1;
+  }
+  if (outl) {
+    for (int c = 0; c < r.n_chunks; ++c)
+      for (int q = 0; q < k; ++q) {
+        const float v = r.topv_part[((int64_t)c * n_rows + i) * k + q];
+        if (v > tv[k - 1]) topk_insert<KMAX>(tv, ti, k, v, r.topi_part[((int64_t)c * n_rows + i) * k + q]);
+      }
+  }
+  for (int q = 0; q < KMAX; ++q)
+    if (ti[q] >= 0) ti[q] = (int32_t)(r.idx_base + (r.idx_map ? r.idx_map[ti[q]] : ti[q]));
+}
+
+// One block per (row, job): the O partials summed in chunk order four features at a time, the denominator and the top-k merge.
+// A hard-negative-only row has no softmax term -- its O partials may not even have been written -- so its osum row is zero.
+__global__ void __launch_bounds__(128) head_reduce_kernel(const ReduceJobs jobs, int n_rows, int D, int k, const uint8_t* __restrict__ is_out) {
   const ReduceJob& r = jobs.j[blockIdx.y];
   const int i = blockIdx.x;
   const int n_chunks = r.n_chunks;
-  const bool no_o = is_out[i] != 0;      // a hard-negative-only row has no softmax term: its O partials may not even have been written
+  const bool no_o = is_out[i] != 0;
   for (int d = threadIdx.x * 4; d < D; d += blockDim.x * 4) {
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
     for (int c = 0; c < n_chunks && !no_o; ++c) {
@@ -540,27 +530,18 @@ __global__ void __launch_bounds__(128) head_reduce_multi_kernel(const ReduceJobs
     *reinterpret_cast<float4*>(r.osum + (int64_t)i * D + d) = acc;
   }
   if (threadIdx.x == 96) {      // scalar part (denominator, top-k merge) on one lane of the last warp
-    float acc = 0.f;
-    for (int c = 0; c < n_chunks; ++c) acc += r.l_part[(int64_t)c * n_rows + i];
-    r.lsum[i] = acc;
-    float tv[KMAX];
-    int32_t ti[KMAX];
-    for (int q = 0; q < KMAX; ++q) {
-      tv[q] = -INFINITY;
-      ti[q] = -1;
-    }
-    if (is_out[i]) {
-      for (int c = 0; c < n_chunks; ++c)
-        for (int q = 0; q < k; ++q) {
-          const float v = r.topv_part[((int64_t)c * n_rows + i) * k + q];
-          if (v > tv[k - 1]) topk_insert<KMAX>(tv, ti, k, v, r.topi_part[((int64_t)c * n_rows + i) * k + q]);
+    r.lsum[i] = chunk_lsum(r, n_rows, i);
+    if (r.topv) {
+      float tv[KMAX];
+      int32_t ti[KMAX];
+      chunk_topk(r, n_rows, k, i, no_o, tv, ti);
+#pragma unroll
+      for (int q = 0; q < KMAX; ++q) {
+        if (q < k) {
+          r.topv[(int64_t)i * k + q] = tv[q];
+          r.topi[(int64_t)i * k + q] = ti[q];
         }
-    }
-    for (int q = 0; q < k; ++q) {
-      r.topv[(int64_t)i * k + q] = tv[q];
-      int32_t id = ti[q];
-      if (id >= 0) id = (int32_t)(r.idx_base + (r.idx_map ? r.idx_map[id] : id));   // -> global slot
-      r.topi[(int64_t)i * k + q] = id;
+      }
     }
   }
 }
@@ -572,17 +553,12 @@ struct FinalizeArgs {
   const float* P;              // [n][D]  (fp32 embeddings; only for nothing but kept for symmetry)
   const float* qf;             // [2][q_local][D]
   const __nv_bfloat16* qh;
-  int use_bf16_rows;           // gather W rows from the bf16 mirror (consistent with the tensor-core sweep)
+  int use_bf16_rows;           // gather W rows from the bf16 mirror (consistent with the tensor-core sweep), else from qf (check mode)
   const int32_t* label;
   const int32_t* tcol;
   const int32_t* tpos;
   const uint8_t* is_out;
   const int32_t* counts;
-  const float* lsum;           // [4][n]
-  const float* osum;           // [4][n][D]
-  const float* tgt;            // [4][n]
-  const float* topv;           // [n_ranks][3][n][k]
-  const int32_t* topi;
   int n_ranks;
   int n, D, k;
   int64_t q_local, col_offset;
@@ -613,15 +589,10 @@ struct FinalizeArgs {
   int64_t dp_slot_off;
 };
 
-__device__ __forceinline__ float w_elem(const FinalizeArgs& a, int r, int64_t local_slot, int d) {
-  const int64_t off = ((int64_t)r * a.q_local + local_slot) * a.D + d;
-  return a.use_bf16_rows ? __bfloat162float(a.qh[off]) : a.qf[off];
-}
-
 // The scalar part of finalize for one row: margin function, log/exp in fp64, top-k merge.  `lsum_at(slot)` returns the row's
 // softmax denominator of stats slot 0..3, `top_at(r, set, q, v, idx)` the q-th top-k candidate of rank r / column set `set`.
-// T = double: the check mode and the statistics-in-the-middle path (1e-5 parity); T = float: the fused bf16 path, whose tolerance is
-// 1e-2 -- the ~100 dependent operations per row are then 1-2 us of latency instead of the 16 us the fp64 pipe takes.
+// T = double: the Stats source (the check mode's 1e-5 parity); T = float: the Partials and Records sources of the bf16 path, whose
+// tolerance is 1e-2 -- the ~100 dependent operations per row are then 1-2 us of latency instead of the 16 us the fp64 pipe takes.
 template <class T, class LsumF, class TgtF, class TopF>
 __device__ __forceinline__ void row_coef_math(const FinalizeArgs& a, int i, int n_ranks, LsumF lsum_at, TgtF tgt_at, TopF top_at, float& loss_out, float (&cO)[2],
                                               float (&cT)[2], int& nw_out, int32_t* wslot_out, uint8_t* wrow_out) {
@@ -698,31 +669,6 @@ __device__ __forceinline__ void row_coef_math(const FinalizeArgs& a, int i, int 
   nw_out = nw;
 }
 
-// Pass 1, one THREAD per row: the scalar part of finalize.  Doing this per thread instead of on thread 0 of a per-row block
-// keeps the fp64 transcendental latency off the critical path.
-__global__ void __launch_bounds__(128) head_row_coef_kernel(const FinalizeArgs a, float* __restrict__ coef, int32_t* __restrict__ nslot,
-                                                            int32_t* __restrict__ wslot, uint8_t* __restrict__ wrow) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  const int n = a.n, k = a.k;
-  if (i >= n) return;
-  float loss, cO[2], cT[2];
-  int nw;
-  row_coef_math<double>(
-      a, i, a.n_ranks, [&](int slot) { return a.lsum[slot * n + i]; }, [&](int l) { return a.tgt[l * n + i]; },
-      [&](int r, int set, int q, float& v, int32_t& idx) {
-        const int64_t base = ((((int64_t)r * 3 + set) * n) + i) * k;
-        v = a.topv[base + q];
-        idx = a.topi[base + q];
-      },
-      loss, cO, cT, nw, wslot + (int64_t)i * 2 * KMAX, wrow + (int64_t)i * 2 * KMAX);
-  a.row_loss[i] = loss;
-  coef[0 * n + i] = cO[0];
-  coef[1 * n + i] = cO[1];
-  coef[2 * n + i] = cT[0];
-  coef[3 * n + i] = cT[1];
-  nslot[i] = nw;
-}
-
 // Per-rank record exchanged by the sharded head (4-byte words, n = rows, k = top-k):
 //   [0, 8n)          float  red[8][n]     lsum slots 0..3 (common loss 1, unused, side 0, side 1), tgt slots 0..3
 //   [8n, 8n+3nk)     float  topv[3][n][k]
@@ -730,41 +676,31 @@ __global__ void __launch_bounds__(128) head_row_coef_kernel(const FinalizeArgs a
 __host__ __device__ __forceinline__ int64_t record_words(int64_t n, int64_t k) { return 8 * n + 6 * n * k; }
 
 // Chunk reduction of the three sweeps' SCALAR partials (softmax denominators, top-k candidates) straight into this rank's
-// record; the O partials stay where they are for head_finalize_fused_kernel<true>.  One thread per (row, sweep).
+// record; the O partials stay where they are for head_finalize_fused_kernel<Records>.  One thread per (row, sweep).
 __global__ void __launch_bounds__(128) head_reduce_scalars_kernel(const ReduceJobs jobs, int n, int k, const uint8_t* __restrict__ is_out,
                                                                   float* __restrict__ rec) {
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= 3 * n) return;
   const int i = t / 3, w = t - 3 * i;
   const ReduceJob& r = jobs.j[w];
-  float acc = 0.f;
-  for (int c = 0; c < r.n_chunks; ++c) acc += r.l_part[(int64_t)c * n + i];
-  rec[(int64_t)(w == 0 ? 0 : 1 + w) * n + i] = acc;
+  rec[(int64_t)(w == 0 ? 0 : 1 + w) * n + i] = chunk_lsum(r, n, i);
   if (w == 0) rec[(int64_t)1 * n + i] = 0.f;
   float tv[KMAX];
   int32_t ti[KMAX];
-  for (int q = 0; q < KMAX; ++q) {
-    tv[q] = -INFINITY;
-    ti[q] = -1;
-  }
-  if (is_out[i]) {
-    for (int c = 0; c < r.n_chunks; ++c)
-      for (int q = 0; q < k; ++q) {
-        const float v = r.topv_part[((int64_t)c * n + i) * k + q];
-        if (v > tv[k - 1]) topk_insert<KMAX>(tv, ti, k, v, r.topi_part[((int64_t)c * n + i) * k + q]);
-      }
-  }
+  chunk_topk(r, n, k, i, is_out[i], tv, ti);
   float* topv = rec + 8 * (int64_t)n;
   int32_t* topi = reinterpret_cast<int32_t*>(rec + 8 * (int64_t)n + 3 * (int64_t)n * k);
-  for (int q = 0; q < k; ++q) {
-    int32_t id = ti[q];
-    if (id >= 0) id = (int32_t)(r.idx_base + (r.idx_map ? r.idx_map[id] : id));   // -> global slot
-    topv[((int64_t)w * n + i) * k + q] = tv[q];
-    topi[((int64_t)w * n + i) * k + q] = id;
+#pragma unroll
+  for (int q = 0; q < KMAX; ++q) {
+    if (q < k) {
+      topv[((int64_t)w * n + i) * k + q] = tv[q];
+      topi[((int64_t)w * n + i) * k + q] = ti[q];
+    }
   }
 }
 
-// One prototype row as the fused finalize reads it: the bf16 mirror row, or (overlay) an fp32 row rounded on the fly.
+// One prototype row as finalize reads it: the bf16 mirror row, an fp32 row standing in for it (overlay; rounded on the fly), or in
+// check mode the fp32 queue row itself.
 struct WRow {
   const __nv_bfloat16* h;
   const float* f;
@@ -772,17 +708,23 @@ struct WRow {
 __device__ __forceinline__ WRow w_row(const FinalizeArgs& a, int r, int64_t loc) {
   WRow w;
   const int64_t e = (int64_t)r * a.q_local + loc;
-  w.h = a.qh + e * a.D;
+  w.h = nullptr;
   w.f = nullptr;
+  if (!a.use_bf16_rows) {
+    w.f = a.qf + e * a.D;
+    return w;
+  }
+  w.h = a.qh + e * a.D;
   if (a.ovl_map) {
     const int32_t c = __ldg(a.ovl_map + e);
     if (c >= 0) w.f = (c & 0x40000000) ? a.ovl_undo + (int64_t)(c & 0x3fffffff) * a.D : a.ovl_g + (int64_t)c * a.D;
   }
   return w;
 }
-__device__ __forceinline__ float4 w_load4(const WRow& w, int d) {
+__device__ __forceinline__ float4 w_load4(const WRow& w, int d, bool bf16) {
   if (w.f) {
     const float4 v = *reinterpret_cast<const float4*>(w.f + d);
+    if (!bf16) return v;
     return make_float4(__bfloat162float(__float2bfloat16(v.x)), __bfloat162float(__float2bfloat16(v.y)), __bfloat162float(__float2bfloat16(v.z)),
                        __bfloat162float(__float2bfloat16(v.w)));
   }
@@ -792,141 +734,224 @@ __device__ __forceinline__ float4 w_load4(const WRow& w, int d) {
   return make_float4(a2.x, a2.y, b2.x, b2.y);
 }
 
-// Fast path of the bf16 AM / Arc head: chunk reduction of the three sweeps' partials, the scalar part and dLoss/dp in ONE
-// launch.  No osum round trip through HBM; replaces reduce + row_coef + finalize.  A block takes FR = 4 rows (2 048 blocks at the 8-GPU
-// row count: the partial sums are ~100 MB to read, and it takes that many loads in flight to read them at the HBM rate):
-//   phase 1 (GATHERED = false only): one thread per (row, sweep) sums the chunk denominators and merges the chunk top-k lists;
-//   phase 2: one THREAD per row does the scalar part (margin function, log / exp, top-k merge over ranks) -- in fp32, all rows of
-//            the grid side by side (one lane per row on the fp64 pipe cost 16 us per row, 3.5 waves of it at 8 192 rows);
-//   phase 3: one warp per row, lanes over D: chunk sums of the three O partials, the two prototype rows of the target (or the
-//            hard-negative rows of an outlier row), 16-byte stores -- the bandwidth part, ~(chunks * 3 + 2) * D * 4 bytes per row.
-//   GATHERED = false (one GPU): the scalars are reduced here from the partials as well;
-//   GATHERED = true (sharded head): the scalars come from the n_ranks gathered records (`rec`, `rec_stride` words apart),
-//     summed in rank order on every rank; O is this rank's partial, so dp is this rank's contribution -- stored locally for a
-//     reduce-scatter, or (dp_peer) straight into the owner rank's staging buffer.
-constexpr int FR = 4;
-template <bool GATHERED>
-__global__ void __launch_bounds__(128) head_finalize_fused_kernel(const ReduceJobs jobs, const FinalizeArgs a, const float* __restrict__ rec,
-                                                                  int64_t rec_stride) {
+// Features d..d+3 of row i of a job's O partials summed in chunk order.  The loads of eight chunks are in flight at once: with a
+// serial chunk loop the finalize ran at memory LATENCY (70 us for 2 048 rows x 9 chunks: 37 MB).
+__device__ __forceinline__ float4 chunk_o4(const ReduceJob& rj, int n, int D, int i, int d) {
+  const float* base = rj.o_part + (int64_t)i * D + d;
+  const int64_t cstride = (int64_t)n * D;
+  const int nc = rj.n_chunks;
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+  int c = 0;
+  for (; c + 8 <= nc; c += 8) {
+    float4 v[8];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) v[u] = __ldcs(reinterpret_cast<const float4*>(base + (c + u) * cstride));
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+      acc.x += v[u].x;
+      acc.y += v[u].y;
+      acc.z += v[u].z;
+      acc.w += v[u].w;
+    }
+  }
+  for (; c + 2 <= nc; c += 2) {
+    const float4 v0 = __ldcs(reinterpret_cast<const float4*>(base + c * cstride));
+    const float4 v1 = __ldcs(reinterpret_cast<const float4*>(base + (c + 1) * cstride));
+    acc.x += v0.x;
+    acc.y += v0.y;
+    acc.z += v0.z;
+    acc.w += v0.w;
+    acc.x += v1.x;
+    acc.y += v1.y;
+    acc.z += v1.z;
+    acc.w += v1.w;
+  }
+  for (; c < nc; ++c) {
+    const float4 v = __ldcs(reinterpret_cast<const float4*>(base + c * cstride));
+    acc.x += v.x;
+    acc.y += v.y;
+    acc.z += v.z;
+    acc.w += v.w;
+  }
+  return acc;
+}
+
+// The three sources of head_finalize_fused_kernel's statistics.  Each stages what its rows' scalar part reads (`stage`, all threads
+// of the block), runs that scalar part for row i (`coef`: row_coef_math with the source's lambdas and arithmetic type) and gives the
+// O sum of a stats slot (0 common loss 1, 1 common loss 2, 2 side 0, 3 side 1) for four features (`o4`).  Slot 1 is SV's alone, and
+// only `sv_slot` sources (SV runs the statistics path) hold it: AM / Arc read slot 0 for both losses.
+constexpr int FR = 4;      // rows per block
+
+// One GPU, bf16 AM / Arc (ffc_head_pass_single): the three merged sweeps' chunk partials, reduced here -- one thread per (row, sweep)
+// sums the chunk denominators and merges the chunk top-k lists.  No statistics round trip through HBM.
+struct Partials {
+  static constexpr bool sv_slot = false;
+  ReduceJobs jobs;
+  const float* tgt;            // [4][n] target cosines (prep)
+  struct Smem {
+    float l[FR][3];
+    float tv[FR][3][KMAX];
+    int32_t ti[FR][3][KMAX];
+  };
+  __device__ void stage(const FinalizeArgs& a, int row0, Smem& s) const {
+    const int tid = threadIdx.x;
+    if (tid < FR * 3) {
+      const int r = tid / 3, j = tid - 3 * r, i = row0 + r;
+      if (i < a.n) {
+        const ReduceJob& rj = jobs.j[j];
+        s.l[r][j] = chunk_lsum(rj, a.n, i);
+        float tv[KMAX];
+        int32_t ti[KMAX];
+        chunk_topk(rj, a.n, a.k, i, a.is_out[i], tv, ti);
+        for (int q = 0; q < KMAX; ++q) {
+          s.tv[r][j][q] = tv[q];
+          s.ti[r][j][q] = ti[q];
+        }
+      }
+    }
+    __syncthreads();
+  }
+  __device__ void coef(const FinalizeArgs& a, const Smem& s, int r, int i, float& loss, float (&cO)[2], float (&cT)[2], int& nw, int32_t* wslot,
+                       uint8_t* wrow) const {
+    row_coef_math<float>(
+        a, i, 1, [&](int slot) { return slot == 0 ? s.l[r][0] : (slot >= 2 ? s.l[r][slot - 1] : 0.f); }, [&](int l) { return tgt[l * a.n + i]; },
+        [&](int, int set, int e, float& v, int32_t& idx) {
+          v = s.tv[r][set][e];
+          idx = s.ti[r][set][e];
+        },
+        loss, cO, cT, nw, wslot, wrow);
+  }
+  __device__ float4 o4(const FinalizeArgs& a, int slot, int i, int d) const { return chunk_o4(jobs.j[slot == 0 ? 0 : slot - 1], a.n, a.D, i, d); }
+};
+
+// Sharded bf16 AM / Arc (ffc_head_finalize_gathered_ex): the scalars come from the n_ranks gathered records (`rec`, `stride` words
+// apart), summed in rank order on every rank; O is this rank's partial, so dp is this rank's contribution.  The records are staged
+// through shared memory -- per row 6 scalars x R ranks and, for an outlier row, 3 candidate sets x R ranks x k (value, slot) pairs.
+// Read by the one thread that does the row's scalar part they were ~50 (positive row) / ~500 (outlier row) dependent global loads:
+// the latency of this phase paced the kernel at 8 ranks.
+struct Records {
+  static constexpr bool sv_slot = false;
+  ReduceJobs jobs;
+  const float* rec;
+  int64_t stride;
+  static constexpr int RS = 16;      // ranks the staging is sized for (more: the records are read in place)
+  struct Smem {
+    float red[FR][6][RS];
+    float cv[FR][3][RS][KMAX];
+    int32_t ci[FR][3][RS][KMAX];
+  };
+  __device__ void stage(const FinalizeArgs& a, int row0, Smem& s) const {
+    const int R = a.n_ranks, n = a.n, k = a.k;
+    if (R > RS) return;
+    for (int e = threadIdx.x; e < FR * 6 * R; e += 128) {
+      const int r = e / (6 * R), j = (e / R) % 6, q = e % R, i = row0 + r;
+      if (i < n) s.red[r][j][q] = rec[q * stride + (int64_t)j * n + i];
+    }
+    for (int e = threadIdx.x; e < FR * 3 * R * k; e += 128) {
+      const int r = e / (3 * R * k), set = (e / (R * k)) % 3, q = (e / k) % R, x = e % k, i = row0 + r;
+      if (i < n && a.is_out[i]) {
+        const float* base = rec + q * stride + 8 * (int64_t)n;
+        const int64_t o = ((int64_t)set * n + i) * k + x;
+        s.cv[r][set][q][x] = base[o];
+        s.ci[r][set][q][x] = reinterpret_cast<const int32_t*>(base + 3 * (int64_t)n * k)[o];
+      }
+    }
+    __syncthreads();
+  }
+  __device__ void coef(const FinalizeArgs& a, const Smem& s, int r, int i, float& loss, float (&cO)[2], float (&cT)[2], int& nw, int32_t* wslot,
+                       uint8_t* wrow) const {
+    const int R = a.n_ranks, n = a.n, k = a.k;
+    if (R <= RS) {
+      row_coef_math<float>(
+          a, i, R,
+          [&](int slot) {
+            float acc = 0.f;
+            for (int q = 0; q < R; ++q) acc += s.red[r][slot][q];      // rank order: the same sum on every rank
+            return acc;
+          },
+          [&](int l) {
+            float acc = 0.f;
+            for (int q = 0; q < R; ++q) acc += s.red[r][4 + l][q];
+            return acc;
+          },
+          [&](int q, int set, int e, float& v, int32_t& idx) {
+            v = s.cv[r][set][q][e];
+            idx = s.ci[r][set][q][e];
+          },
+          loss, cO, cT, nw, wslot, wrow);
+    } else {
+      row_coef_math<float>(
+          a, i, R,
+          [&](int slot) {
+            float acc = 0.f;
+            for (int q = 0; q < R; ++q) acc += rec[q * stride + (int64_t)slot * n + i];
+            return acc;
+          },
+          [&](int l) {
+            float acc = 0.f;
+            for (int q = 0; q < R; ++q) acc += rec[q * stride + (int64_t)(4 + l) * n + i];
+            return acc;
+          },
+          [&](int q, int set, int e, float& v, int32_t& idx) {
+            const float* base = rec + q * stride + 8 * (int64_t)n;
+            const int64_t o = ((int64_t)set * n + i) * k + e;
+            v = base[o];
+            idx = reinterpret_cast<const int32_t*>(base + 3 * (int64_t)n * k)[o];
+          },
+          loss, cO, cT, nw, wslot, wrow);
+    }
+  }
+  __device__ float4 o4(const FinalizeArgs& a, int slot, int i, int d) const { return chunk_o4(jobs.j[slot == 0 ? 0 : slot - 1], a.n, a.D, i, d); }
+};
+
+// ffc_head_sweep + ffc_head_finalize (fp32 check mode, SV, several GPUs through the statistics): the reduced statistics, after the
+// caller's all-reduce / all-gather.
+struct Stats {
+  static constexpr bool sv_slot = true;
+  ffc_head_stats st;
+  struct Smem {};
+  __device__ void stage(const FinalizeArgs&, int, Smem&) const {}
+  __device__ void coef(const FinalizeArgs& a, const Smem&, int, int i, float& loss, float (&cO)[2], float (&cT)[2], int& nw, int32_t* wslot,
+                       uint8_t* wrow) const {
+    const int n = a.n, k = a.k;
+    row_coef_math<double>(
+        a, i, a.n_ranks, [&](int slot) { return st.lsum[slot * n + i]; }, [&](int l) { return st.tgt[l * n + i]; },
+        [&](int r, int set, int q, float& v, int32_t& idx) {
+          const int64_t base = ((((int64_t)r * 3 + set) * n) + i) * k;
+          v = st.topv[base + q];
+          idx = st.topi[base + q];
+        },
+        loss, cO, cT, nw, wslot, wrow);
+  }
+  __device__ float4 o4(const FinalizeArgs& a, int slot, int i, int d) const {
+    return *reinterpret_cast<const float4*>(st.osum + ((int64_t)slot * a.n + i) * a.D + d);
+  }
+};
+
+// Finalize of every head configuration in ONE launch.  A block takes FR = 4 rows (2 048 blocks at the 8-GPU row count: the partial
+// sums are ~100 MB to read, and it takes that many loads in flight to read them at the HBM rate):
+//   stage:   the source brings its rows' scalar inputs into shared memory;
+//   phase 2: one THREAD per row does the scalar part (margin function, log / exp, top-k merge over ranks), all rows of the grid side by
+//            side;
+//   phase 3: (row, 4 features) items dealt to the 128 threads: the O sums, the two prototype rows of the target (or the hard-negative
+//            rows of an outlier row), 16-byte stores -- the bandwidth part.  dp is stored locally or, on a shard (dp_peer), straight into
+//            the owner rank's staging buffer.
+template <class Src>
+__global__ void __launch_bounds__(128) head_finalize_fused_kernel(const Src src, const FinalizeArgs a) {
   const int tid = threadIdx.x;
-  const int row0 = blockIdx.x * FR, n = a.n, D = a.D, k = a.k;
-  __shared__ float s_l[FR][3];
-  __shared__ float s_tv[FR][3][KMAX];
-  __shared__ int32_t s_ti[FR][3][KMAX];
+  const int row0 = blockIdx.x * FR, n = a.n, D = a.D;
+  __shared__ typename Src::Smem s_src;
   __shared__ float s_coef[FR][4];
   __shared__ int s_nw[FR];
   __shared__ int32_t s_wslot[FR][2 * KMAX];
   __shared__ uint8_t s_wrow[FR][2 * KMAX];
   __shared__ WRow s_t0[FR], s_t1[FR];
-  if (!GATHERED) {
-    if (tid < FR * 3) {
-      const int r = tid / 3, j = tid - 3 * r, i = row0 + r;
-      if (i < n) {
-        const ReduceJob& rj = jobs.j[j];
-        float acc = 0.f;
-        for (int c = 0; c < rj.n_chunks; ++c) acc += rj.l_part[(int64_t)c * n + i];
-        s_l[r][j] = acc;
-        float tv[KMAX];
-        int32_t ti[KMAX];
-        for (int q = 0; q < KMAX; ++q) {
-          tv[q] = -INFINITY;
-          ti[q] = -1;
-        }
-        if (a.is_out[i]) {
-          for (int c = 0; c < rj.n_chunks; ++c)
-            for (int q = 0; q < k; ++q) {
-              const float v = rj.topv_part[((int64_t)c * n + i) * k + q];
-              if (v > tv[k - 1]) topk_insert<KMAX>(tv, ti, k, v, rj.topi_part[((int64_t)c * n + i) * k + q]);
-            }
-        }
-        for (int q = 0; q < KMAX; ++q) {
-          int32_t id = ti[q];
-          if (id >= 0) id = (int32_t)(rj.idx_base + (rj.idx_map ? rj.idx_map[id] : id));   // -> global slot
-          s_tv[r][j][q] = tv[q];
-          s_ti[r][j][q] = id;
-        }
-      }
-    }
-    __syncthreads();
-  }
-  // GATHERED: the ranks' records are staged through shared memory by all threads -- per row 6 scalars x R ranks and, for an outlier
-  // row, 3 candidate sets x R ranks x k (value, slot) pairs.  Read by the one thread that does the row's scalar part they were
-  // ~50 (positive row) / ~500 (outlier row) dependent global loads: the latency of this phase paced the kernel at 8 ranks.
-  constexpr int RS = 16;                       // ranks the staging is sized for (more: the records are read in place)
-  __shared__ float s_red[GATHERED ? FR : 1][6][GATHERED ? RS : 1];
-  __shared__ float s_cv[GATHERED ? FR : 1][3][GATHERED ? RS : 1][KMAX];
-  __shared__ int32_t s_ci[GATHERED ? FR : 1][3][GATHERED ? RS : 1][KMAX];
-  const bool staged = GATHERED && a.n_ranks <= RS;
-  if (staged) {
-    const int R = a.n_ranks;
-    for (int e = tid; e < FR * 6 * R; e += 128) {
-      const int r = e / (6 * R), j = (e / R) % 6, q = e % R, i = row0 + r;
-      if (i < n) s_red[r][j][q] = rec[q * rec_stride + (int64_t)j * n + i];
-    }
-    for (int e = tid; e < FR * 3 * R * k; e += 128) {
-      const int r = e / (3 * R * k), set = (e / (R * k)) % 3, q = (e / k) % R, x = e % k, i = row0 + r;
-      if (i < n && a.is_out[i]) {
-        const float* base = rec + q * rec_stride + 8 * (int64_t)n;
-        const int64_t o = ((int64_t)set * n + i) * k + x;
-        s_cv[r][set][q][x] = base[o];
-        s_ci[r][set][q][x] = reinterpret_cast<const int32_t*>(base + 3 * (int64_t)n * k)[o];
-      }
-    }
-    __syncthreads();
-  }
+  src.stage(a, row0, s_src);
   if (tid < FR && row0 + tid < n) {
     const int r = tid, i = row0 + r;
     float loss, cO[2], cT[2];
     int nw;
-    if (staged) {
-      const int R = a.n_ranks;
-      row_coef_math<float>(
-          a, i, R,
-          [&](int slot) {
-            float acc = 0.f;
-            for (int q = 0; q < R; ++q) acc += s_red[r][slot][q];      // rank order: the same sum on every rank
-            return acc;
-          },
-          [&](int l) {
-            float acc = 0.f;
-            for (int q = 0; q < R; ++q) acc += s_red[r][4 + l][q];
-            return acc;
-          },
-          [&](int q, int set, int e, float& v, int32_t& idx) {
-            v = s_cv[r][set][q][e];
-            idx = s_ci[r][set][q][e];
-          },
-          loss, cO, cT, nw, s_wslot[r], s_wrow[r]);
-    } else if (GATHERED) {
-      const int R = a.n_ranks;
-      row_coef_math<float>(
-          a, i, R,
-          [&](int slot) {
-            float acc = 0.f;
-            for (int q = 0; q < R; ++q) acc += rec[q * rec_stride + (int64_t)slot * n + i];
-            return acc;
-          },
-          [&](int l) {
-            float acc = 0.f;
-            for (int q = 0; q < R; ++q) acc += rec[q * rec_stride + (int64_t)(4 + l) * n + i];
-            return acc;
-          },
-          [&](int q, int set, int e, float& v, int32_t& idx) {
-            const float* base = rec + q * rec_stride + 8 * (int64_t)n;
-            const int64_t o = ((int64_t)set * n + i) * k + e;
-            v = base[o];
-            idx = reinterpret_cast<const int32_t*>(base + 3 * (int64_t)n * k)[o];
-          },
-          loss, cO, cT, nw, s_wslot[r], s_wrow[r]);
-    } else {
-      row_coef_math<float>(
-          a, i, 1, [&](int slot) { return slot == 0 ? s_l[r][0] : (slot >= 2 ? s_l[r][slot - 1] : 0.f); }, [&](int l) { return a.tgt[l * n + i]; },
-          [&](int, int set, int e, float& v, int32_t& idx) {
-            v = s_tv[r][set][e];
-            idx = s_ti[r][set][e];
-          },
-          loss, cO, cT, nw, s_wslot[r], s_wrow[r]);
-    }
+    src.coef(a, s_src, r, i, loss, cO, cT, nw, s_wslot[r], s_wrow[r]);
     a.row_loss[i] = loss;
     s_coef[r][0] = cO[0];
     s_coef[r][1] = cO[1];
@@ -959,11 +984,7 @@ __global__ void __launch_bounds__(128) head_finalize_fused_kernel(const ReduceJo
     s_t1[tid] = t1;
   }
   __syncthreads();
-  // phase 3: (row, 4 features) items dealt to the 128 threads; the chunk loads of an item are independent (issued eight at a time,
-  // added in chunk order) -- with one warp per row and a serial chunk loop the kernel ran at memory LATENCY (70 us for 2 048 rows x
-  // 9 chunks: 37 MB)
   const int D4 = D >> 2;
-  const int64_t cstride = (int64_t)n * D;
   for (int item = tid; item < FR * D4; item += 128) {
     const int r = item / D4, d = (item - r * D4) * 4;
     const int i = row0 + r;
@@ -973,55 +994,15 @@ __global__ void __launch_bounds__(128) head_finalize_fused_kernel(const ReduceJo
     float g[4] = {0.f, 0.f, 0.f, 0.f};
     if (!outl) {
       const float cO0 = s_coef[r][0], cO1 = s_coef[r][1], cT0 = s_coef[r][2], cT1 = s_coef[r][3];
-      float o[3][4];
-#pragma unroll
-      for (int jb = 0; jb < 3; ++jb) {
-        const ReduceJob& rj = jobs.j[jb];
-        const float* base = rj.o_part + (int64_t)i * D + d;
-        const int nc = rj.n_chunks;
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-        int c = 0;
-        for (; c + 8 <= nc; c += 8) {
-          float4 v[8];
-#pragma unroll
-          for (int u = 0; u < 8; ++u) v[u] = __ldcs(reinterpret_cast<const float4*>(base + (c + u) * cstride));
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            acc.x += v[u].x;
-            acc.y += v[u].y;
-            acc.z += v[u].z;
-            acc.w += v[u].w;
-          }
-        }
-        for (; c + 2 <= nc; c += 2) {
-          const float4 v0 = __ldcs(reinterpret_cast<const float4*>(base + c * cstride));
-          const float4 v1 = __ldcs(reinterpret_cast<const float4*>(base + (c + 1) * cstride));
-          acc.x += v0.x;
-          acc.y += v0.y;
-          acc.z += v0.z;
-          acc.w += v0.w;
-          acc.x += v1.x;
-          acc.y += v1.y;
-          acc.z += v1.z;
-          acc.w += v1.w;
-        }
-        for (; c < nc; ++c) {
-          const float4 v = __ldcs(reinterpret_cast<const float4*>(base + c * cstride));
-          acc.x += v.x;
-          acc.y += v.y;
-          acc.z += v.z;
-          acc.w += v.w;
-        }
-        o[jb][0] = acc.x;
-        o[jb][1] = acc.y;
-        o[jb][2] = acc.z;
-        o[jb][3] = acc.w;
-      }
-#pragma unroll
-      for (int e = 0; e < 4; ++e) g[e] = cO0 * (o[0][e] + o[1][e]) + cO1 * (o[0][e] + o[2][e]);
+      const float4 oc0 = src.o4(a, 0, i, d), os0 = src.o4(a, 2, i, d), os1 = src.o4(a, 3, i, d);
+      const float4 oc1 = Src::sv_slot && a.loss_type == FFC_LOSS_SV ? src.o4(a, 1, i, d) : oc0;
+      g[0] = cO0 * (oc0.x + os0.x) + cO1 * (oc1.x + os1.x);
+      g[1] = cO0 * (oc0.y + os0.y) + cO1 * (oc1.y + os1.y);
+      g[2] = cO0 * (oc0.z + os0.z) + cO1 * (oc1.z + os1.z);
+      g[3] = cO0 * (oc0.w + os0.w) + cO1 * (oc1.w + os1.w);
       const WRow t0 = s_t0[r], t1 = s_t1[r];
-      if (t0.h) {
-        const float4 w0 = w_load4(t0, d), w1 = w_load4(t1, d);
+      if (t0.h || t0.f) {
+        const float4 w0 = w_load4(t0, d, a.use_bf16_rows), w1 = w_load4(t1, d, a.use_bf16_rows);
         g[0] += cT0 * w0.x + cT1 * w1.x;
         g[1] += cT0 * w0.y + cT1 * w1.y;
         g[2] += cT0 * w0.z + cT1 * w1.z;
@@ -1033,7 +1014,7 @@ __global__ void __launch_bounds__(128) head_finalize_fused_kernel(const ReduceJo
       for (int x = 0; x < nw; ++x) {
         const int64_t loc = (int64_t)s_wslot[r][x] - a.col_offset;
         if (loc >= 0 && loc < a.q_local) {
-          const float4 wv = w_load4(w_row(a, s_wrow[r][x], loc), d);
+          const float4 wv = w_load4(w_row(a, s_wrow[r][x], loc), d, a.use_bf16_rows);
           g[0] += cO0 * wv.x;
           g[1] += cO0 * wv.y;
           g[2] += cO0 * wv.z;
@@ -1046,32 +1027,6 @@ __global__ void __launch_bounds__(128) head_finalize_fused_kernel(const ReduceJo
   // rows stored into a peer's staging buffer: make them visible system-wide before this kernel counts as finished -- the flag that
   // tells the peer "my rows are there" is written by the next launch in the stream (ffc_sum_slabs_barrier)
   if (a.dp_peer) __threadfence_system();
-}
-
-// Pass 2, one block per row: dLoss/dp from the accumulated sums (bandwidth bound).
-__global__ void __launch_bounds__(128) head_finalize_kernel(const FinalizeArgs a, const float* __restrict__ coef, const int32_t* __restrict__ nslot,
-                                                            const int32_t* __restrict__ wslot, const uint8_t* __restrict__ wrow) {
-  const int i = blockIdx.x, n = a.n, D = a.D;
-  const bool outl = a.is_out[i];
-  const float cO0 = coef[0 * n + i], cO1 = coef[1 * n + i], cT0 = coef[2 * n + i], cT1 = coef[3 * n + i];
-  const int32_t tc = a.tcol[i];
-  const int trow2 = (a.tpos[i] >= 0) ? 1 : 0;
-  const int nw = nslot[i];
-  for (int d = threadIdx.x; d < D; d += blockDim.x) {
-    float g = 0.f;
-    if (!outl) {
-      const float oc0 = a.osum[((int64_t)0 * n + i) * D + d];
-      const float oc1 = a.loss_type == FFC_LOSS_SV ? a.osum[((int64_t)1 * n + i) * D + d] : oc0;
-      g = cO0 * (oc0 + a.osum[((int64_t)2 * n + i) * D + d]) + cO1 * (oc1 + a.osum[((int64_t)3 * n + i) * D + d]);
-      if (tc >= 0) g += cT0 * w_elem(a, 0, tc, d) + cT1 * w_elem(a, trow2, tc, d);
-    } else {
-      for (int e = 0; e < nw; ++e) {
-        const int64_t loc = (int64_t)wslot[(int64_t)i * 2 * KMAX + e] - a.col_offset;
-        if (loc >= 0 && loc < a.q_local) g += cO0 * w_elem(a, wrow[(int64_t)i * 2 * KMAX + e], loc, d);
-      }
-    }
-    a.dp[(int64_t)i * D + d] = g;
-  }
 }
 
 __global__ void __launch_bounds__(1024) head_loss_sum_kernel(const float* __restrict__ row_loss, int n, float* loss_out) {
@@ -1204,6 +1159,44 @@ extern "C" int ffc_head_destroy(ffc_head_t* h) {
   return FFC_OK;
 }
 
+// The reduce job of one sweep: its chunk partials -> stats slot `stat_slot` (lsum / osum) and top-k slot `top_slot` (-1: none), the
+// candidates' columns mapped to global slots by idx_base + idx_map[col] (idx_map NULL: the column itself).
+static ReduceJob reduce_job(const SweepArgs& w, const ffc_head_stats* out, int stat_slot, int top_slot, int64_t idx_base, const int32_t* idx_map) {
+  const int64_t n = w.n_rows, D = w.D, k = w.k;
+  ReduceJob r;
+  r.l_part = w.l_part;
+  r.o_part = w.o_part;
+  r.topv_part = w.topv_part;
+  r.topi_part = w.topi_part;
+  r.n_chunks = w.n_chunks;
+  r.lsum = out->lsum + stat_slot * n;
+  r.osum = out->osum + stat_slot * n * D;
+  r.topv = top_slot >= 0 ? out->topv + top_slot * n * k : nullptr;
+  r.topi = top_slot >= 0 ? out->topi + top_slot * n * k : nullptr;
+  r.idx_base = idx_base;
+  r.idx_map = idx_map;
+  return r;
+}
+
+// `launch()` between a pair of timing events (ffc_head_set_timing / ffc_head_get_timing) when `timed`.
+template <class F>
+static int timed_launch(ffc_head* h, bool timed, cudaStream_t s, F launch) {
+  if (!timed) return launch();
+  if (h->ev_used + 2 > h->ev->size()) {
+    for (int e = 0; e < 2; ++e) {
+      cudaEvent_t ev;
+      FFC_CUDA(cudaEventCreate(&ev));
+      h->ev->push_back(ev);
+    }
+  }
+  FFC_CUDA(cudaEventRecord((*h->ev)[h->ev_used], s));
+  const int rc = launch();
+  if (rc) return rc;
+  FFC_CUDA(cudaEventRecord((*h->ev)[h->ev_used + 1], s));
+  h->ev_used += 2;
+  return FFC_OK;
+}
+
 static int run_one_sweep(ffc_head* h, SweepArgs a, int cache_slot, int stat_slot, int top_slot, const ffc_head_stats* out, int64_t idx_base,
                          const int32_t* idx_map, cudaStream_t s) {
   const bool bf16 = h->cfg.precision == FFC_PREC_BF16;
@@ -1214,27 +1207,12 @@ static int run_one_sweep(ffc_head* h, SweepArgs a, int cache_slot, int stat_slot
   a.o_part = h->o_part;
   a.topv_part = h->topv_part;
   a.topi_part = h->topi_part;
-  const bool timed = h->timing && cache_slot == 0;
-  if (timed) {
-    if (h->ev_used + 2 > h->ev->size()) {
-      for (int e = 0; e < 2; ++e) {
-        cudaEvent_t ev;
-        FFC_CUDA(cudaEventCreate(&ev));
-        h->ev->push_back(ev);
-      }
-    }
-    FFC_CUDA(cudaEventRecord((*h->ev)[h->ev_used], s));
-  }
-  int rc = bf16 ? launch_sweep_sm100(h->sm100, cache_slot, a, s) : launch_sweep_simt(a, s);
+  int rc = timed_launch(h, h->timing && cache_slot == 0, s, [&] { return bf16 ? launch_sweep_sm100(h->sm100, cache_slot, a, s) : launch_sweep_simt(a, s); });
   if (rc) return rc;
-  if (timed) {
-    FFC_CUDA(cudaEventRecord((*h->ev)[h->ev_used + 1], s));
-    h->ev_used += 2;
-  }
-  const int n = a.n_rows, D = a.D, k = a.k;
-  head_reduce_kernel<<<n, 128, 0, s>>>(a.l_part, a.o_part, a.topv_part, a.topi_part, a.n_chunks, n, D, k, out->lsum + (int64_t)stat_slot * n,
-                                       out->osum + (int64_t)stat_slot * n * D, top_slot >= 0 ? out->topv + (int64_t)top_slot * n * k : nullptr,
-                                       top_slot >= 0 ? out->topi + (int64_t)top_slot * n * k : nullptr, a.is_out, idx_base, idx_map);
+  ReduceJobs jobs;
+  jobs.j[0] = reduce_job(a, out, stat_slot, top_slot, idx_base, idx_map);
+  jobs.n = 1;
+  head_reduce_kernel<<<dim3(a.n_rows, jobs.n), 128, 0, s>>>(jobs, a.n_rows, a.D, a.k, a.is_out);
   FFC_LAUNCH_CHECK();
   return FFC_OK;
 }
@@ -1246,6 +1224,7 @@ static int run_merged_sweeps(ffc_head* h, SweepArgs a, const ffc_head_pass* in, 
   const int n = a.n_rows, D = a.D, k = a.k;
   SweepArgs sw[3];
   ReduceJobs jobs;
+  jobs.n = 3;
   int64_t part_row = 0;
   for (int i = 0; i < 3; ++i) {
     SweepArgs& w = sw[i];
@@ -1270,44 +1249,17 @@ static int run_merged_sweeps(ffc_head* h, SweepArgs a, const ffc_head_pass* in, 
     w.o_part = h->o_part + part_row * D;
     w.topv_part = h->topv_part + part_row * k;
     w.topi_part = h->topi_part + part_row * k;
-    const int stat_slot = i == 0 ? 0 : 1 + i, top_slot = i;
-    ReduceJob& r = jobs.j[i];
-    r.l_part = w.l_part;
-    r.o_part = w.o_part;
-    r.topv_part = w.topv_part;
-    r.topi_part = w.topi_part;
-    r.n_chunks = w.n_chunks;
-    r.lsum = out->lsum + (int64_t)stat_slot * n;
-    r.osum = out->osum + (int64_t)stat_slot * n * D;
-    r.topv = out->topv + (int64_t)top_slot * n * k;
-    r.topi = out->topi + (int64_t)top_slot * n * k;
-    r.idx_base = c.col_offset;
-    r.idx_map = i == 0 ? nullptr : in->ones_list;
+    jobs.j[i] = reduce_job(w, out, i == 0 ? 0 : 1 + i, i, c.col_offset, i == 0 ? nullptr : in->ones_list);
     part_row += (int64_t)w.n_chunks * n;
   }
   FFC_REQUIRE(part_row <= h->part_rows_cap && sw[0].n_chunks <= h->max_chunks, "head sweep: partial workspace too small (%d chunks x %d rows)",
               sw[0].n_chunks, n);
-  const bool timed = h->timing != 0;
-  if (timed) {
-    if (h->ev_used + 2 > h->ev->size()) {
-      for (int e = 0; e < 2; ++e) {
-        cudaEvent_t ev;
-        FFC_CUDA(cudaEventCreate(&ev));
-        h->ev->push_back(ev);
-      }
-    }
-    FFC_CUDA(cudaEventRecord((*h->ev)[h->ev_used], s));
-  }
-  int rc = launch_sweeps_sm100(h->sm100, sw, 3, s);
+  int rc = timed_launch(h, h->timing != 0, s, [&] { return launch_sweeps_sm100(h->sm100, sw, 3, s); });
   if (rc) return rc;
-  if (timed) {
-    FFC_CUDA(cudaEventRecord((*h->ev)[h->ev_used + 1], s));
-    h->ev_used += 2;
-  }
   *h->jobs = jobs;
   h->jobs_pending = defer_reduce ? 1 : 0;
   if (!defer_reduce) {
-    head_reduce_multi_kernel<<<dim3(n, 3), 128, 0, s>>>(jobs, n, D, k, a.is_out);
+    head_reduce_kernel<<<dim3(n, jobs.n), 128, 0, s>>>(jobs, n, D, k, a.is_out);
     FFC_LAUNCH_CHECK();
   }
   return FFC_OK;
@@ -1347,6 +1299,7 @@ static int head_sweep_impl(ffc_head_t* h, const ffc_head_pass* in, const ffc_hea
   FFC_REQUIRE(n >= 1 && n <= c.max_rows, "ffc_head_sweep: n_rows=%d outside [1,%d]", n, c.max_rows);
   FFC_REQUIRE(in->p_f32 && in->queue_f32 && in->label && in->n_ones && in->ones_list, "ffc_head_sweep: NULL input");
   FFC_REQUIRE(out->lsum && out->osum && out->tgt && out->topv && out->topi, "ffc_head_sweep: NULL stats");
+  FFC_REQUIRE(((uintptr_t)out->osum & 15) == 0, "ffc_head_sweep: osum must be 16-byte aligned");
   const bool bf16 = c.precision == FFC_PREC_BF16;
   FFC_REQUIRE(!bf16 || in->queue_bf16, "ffc_head_sweep: the bf16 path needs the bf16 queue mirror");
   cudaStream_t s = (cudaStream_t)stream;
@@ -1454,7 +1407,7 @@ extern "C" int ffc_head_finalize(ffc_head_t* h, const ffc_head_pass* in, const f
   return head_finalize_impl(h, in, stats, n_ranks_topk, loss_out, dp_out, stream);
 }
 
-static FinalizeArgs make_finalize_args(ffc_head_t* h, const ffc_head_pass* in, const ffc_head_stats* stats, int n_ranks, float* dp_out) {
+static FinalizeArgs make_finalize_args(ffc_head_t* h, const ffc_head_pass* in, int n_ranks, float* dp_out) {
   const ffc_head_config& c = h->cfg;
   FinalizeArgs a;
   memset(&a, 0, sizeof(a));
@@ -1467,13 +1420,6 @@ static FinalizeArgs make_finalize_args(ffc_head_t* h, const ffc_head_pass* in, c
   a.tpos = h->tpos;
   a.is_out = h->is_out;
   a.counts = h->counts + 2 * h->pass_parity;
-  if (stats) {
-    a.lsum = stats->lsum;
-    a.osum = stats->osum;
-    a.tgt = stats->tgt;
-    a.topv = stats->topv;
-    a.topi = stats->topi;
-  }
   a.n_ranks = n_ranks;
   a.n = in->n_rows;
   a.D = c.feat_dim;
@@ -1501,19 +1447,17 @@ static int head_finalize_impl(ffc_head_t* h, const ffc_head_pass* in, const ffc_
                               void* stream) {
   FFC_REQUIRE(h && in && stats && loss_out && dp_out, "ffc_head_finalize: NULL argument");
   FFC_REQUIRE(n_ranks_topk >= 1, "ffc_head_finalize: n_ranks_topk must be >= 1");
+  FFC_REQUIRE((((uintptr_t)stats->osum | (uintptr_t)dp_out) & 15) == 0, "ffc_head_finalize: osum and dp_out must be 16-byte aligned");
   cudaStream_t s = (cudaStream_t)stream;
-  const FinalizeArgs a = make_finalize_args(h, in, stats, n_ranks_topk, dp_out);
+  const FinalizeArgs a = make_finalize_args(h, in, n_ranks_topk, dp_out);
   if (h->jobs_pending) {       // one-GPU fast path: the sweep left its partials for the fused reduce + finalize
     FFC_REQUIRE(n_ranks_topk == 1, "fused finalize is single-rank");
     h->jobs_pending = 0;
-    head_finalize_fused_kernel<false><<<(a.n + FR - 1) / FR, 128, 0, s>>>(*h->jobs, a, nullptr, 0);
-    FFC_LAUNCH_CHECK();
+    head_finalize_fused_kernel<<<(a.n + FR - 1) / FR, 128, 0, s>>>(Partials{*h->jobs, stats->tgt}, a);
   } else {
-    head_row_coef_kernel<<<(a.n + 127) / 128, 128, 0, s>>>(a, h->coef, h->nslot, h->wslot, h->wrow);
-    FFC_LAUNCH_CHECK();
-    head_finalize_kernel<<<a.n, 128, 0, s>>>(a, h->coef, h->nslot, h->wslot, h->wrow);
-    FFC_LAUNCH_CHECK();
+    head_finalize_fused_kernel<<<(a.n + FR - 1) / FR, 128, 0, s>>>(Stats{*stats}, a);
   }
+  FFC_LAUNCH_CHECK();
   head_loss_sum_kernel<<<1, 1024, 0, s>>>(h->row_loss, a.n, loss_out);
   FFC_LAUNCH_CHECK();
   return FFC_OK;
@@ -1594,7 +1538,7 @@ extern "C" int ffc_head_finalize_gathered_ex(ffc_head_t* h, const ffc_head_pass*
   FFC_REQUIRE(h->jobs_pending, "ffc_head_finalize_gathered: no ffc_head_sweep_record pending");
   FFC_REQUIRE(record_stride_words >= record_words(in->n_rows, h->cfg.topk), "ffc_head_finalize_gathered: record stride too small");
   cudaStream_t s = (cudaStream_t)stream;
-  FinalizeArgs a = make_finalize_args(h, in, nullptr, n_ranks, dp_out);
+  FinalizeArgs a = make_finalize_args(h, in, n_ranks, dp_out);
   if (opts) {
     FFC_REQUIRE(!opts->overlay_map || (opts->overlay_g && opts->overlay_undo), "ffc_head_finalize_gathered_ex: overlay map without its row tables");
     FFC_REQUIRE(!opts->dp_peer || opts->dp_rows_per_rank >= 1, "ffc_head_finalize_gathered_ex: dp_rows_per_rank must be >= 1");
@@ -1606,7 +1550,7 @@ extern "C" int ffc_head_finalize_gathered_ex(ffc_head_t* h, const ffc_head_pass*
     a.dp_slot_off = opts->dp_slot_offset;
   }
   h->jobs_pending = 0;
-  head_finalize_fused_kernel<true><<<(a.n + FR - 1) / FR, 128, 0, s>>>(*h->jobs, a, (const float*)records, record_stride_words);
+  head_finalize_fused_kernel<<<(a.n + FR - 1) / FR, 128, 0, s>>>(Records{*h->jobs, (const float*)records, record_stride_words}, a);
   FFC_LAUNCH_CHECK();
   head_loss_sum_kernel<<<1, 1024, 0, s>>>(h->row_loss, a.n, loss_out);
   FFC_LAUNCH_CHECK();
