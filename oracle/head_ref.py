@@ -55,7 +55,7 @@ def add_margin(cos_theta, label, loss_type, margin, scale, k, mask_svfc=1.2):
         if loss_type != 'AM':
             z = z.float() if z.dtype in (torch.float16, torch.bfloat16) else z
         tgt = label[pos_rows]
-        ar = torch.arange(z.shape[0])
+        ar = torch.arange(z.shape[0], device=z.device)
         gt = z[ar, tgt].view(-1, 1)
         if loss_type == 'AM':
             new_t = gt - margin
@@ -131,7 +131,7 @@ class HeadOracle:
         keep = torch.tensor(sorted(last.values()), dtype=torch.long)
         self.queue[r[keep], c[keep]] = g[keep]
         labels = [self.lru.view(v) for v in pl]             # after this pass's inserts
-        label = torch.tensor(labels, dtype=torch.long)
+        label = torch.tensor(labels, dtype=torch.long, device=self.queue.device)
         w0 = self.queue[0].clone()
         w2 = w0.clone()
         if ones:

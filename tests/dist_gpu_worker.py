@@ -12,7 +12,7 @@ sys.path[:0] = [ROOT, os.path.join(ROOT, 'very-large-scale-face-recognition_b200
 
 def main():
     from ffc_b200.dist import ShardedFFCHead
-    from test_dist_cpu import ShardedOracle
+    from oracle.shard_ref import ShardedOracle
     rank, world, local = int(os.environ['RANK']), int(os.environ['WORLD_SIZE']), int(os.environ['LOCAL_RANK'])
     torch.cuda.set_device(local)
     dev = torch.device('cuda', local)

@@ -124,7 +124,7 @@ def _worker(rank, world, port, loss_type, record_flow, ret):
     dist.init_process_group('gloo', rank=rank, world_size=world)
     try:
         from cpu_shard_backend import CpuShardBackend, CpuShardBackendM
-        from test_dist_cpu import ShardedOracle
+        from oracle.shard_ref import ShardedOracle
         from ffc_b200.dist import ShardedFFCHead
         base = CpuShardBackendM if record_flow else CpuShardBackend
         Backend = type('DqBackend', (DqueueMixin, base), {})

@@ -248,7 +248,7 @@ def _nccl_worker(rank, world, port, loss_type, margin, ret):
     dist.init_process_group('nccl', rank=rank, world_size=world)
     try:
         sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-        from test_dist_cpu import ShardedOracle
+        from oracle.shard_ref import ShardedOracle
         from ffc_b200.dist import ShardedFFCHead
         dev = torch.device('cuda', rank)
         D, Q, B, n_ids = 128, 4099, 64, 3000
