@@ -13,7 +13,8 @@
  *
  * Slots, rows and labels are int32 on the device (the reference uses Python ints / int64 tensors;
  * the Python mirror converts at the boundary).  Keys (identity labels) are int64; the two values
- * INT64_MIN and INT64_MIN+1 are reserved as hash-table sentinels and are rejected.
+ * INT64_MIN and INT64_MIN+1 are reserved as hash-table sentinels and are rejected (ffc_lru_view reports
+ * them absent, ffc_lru_assign raises device flag 5).
  */
 #ifndef FFC_B200_H_
 #define FFC_B200_H_
@@ -28,6 +29,13 @@ extern "C" {
 #define FFC_ERR_INVALID 1
 #define FFC_ERR_CUDA 2
 #define FFC_ERR_STATE 3
+/* A device LRU raises a flag on the device instead of returning an error, because ffc_lru_assign does not synchronise:
+ *   1 = recency ring full, 2 = journal full, 3 = eviction from an empty cache, 4 = candidate scan failed,
+ *   5 = reserved key: a key of the batch is INT64_MIN or INT64_MIN+1 (neither a hit nor a miss).
+ * The next host-sync LRU call (ffc_lru_size, ffc_lru_export) returns FFC_ERR_STATE with the flag in ffc_last_error().
+ * The call that raised it writes cols_out = -1 for the chunk it refused and every later position.  Chunks before it
+ * may have been applied: from the flag until ffc_lru_clear or ffc_lru_import the cache state is unspecified, and
+ * either of those two recovers it. */
 
 #define FFC_LOSS_AM 0  /* ffc.py:73-94  CosFace / additive margin */
 #define FFC_LOSS_ARC 1 /* ffc.py:95-115 ArcFace */
@@ -99,7 +107,7 @@ int ffc_lru_size(ffc_lru_t* h, int64_t* cur_idx_out, int64_t* journal_len_out, v
 /* host-sync: lru.py:102-108 state_dict(): (key, slot) pairs from most to least recently used, into
  * HOST arrays of at least `capacity` entries; *n_out = count. */
 int ffc_lru_export(ffc_lru_t* h, int64_t* keys_host, int32_t* slots_host, int64_t* n_out, void* stream);
-/* host-sync: lru.py:113-128 restore(kvs): requires an empty cache (cur_idx == 0), n <= capacity,
+/* host-sync: lru.py:113-128 restore(kvs): requires an empty cache (cur_idx == 0) or one whose device error flag is set, n <= capacity,
  * distinct keys and distinct slots in [0, capacity). pairs are most- to least-recent. */
 int ffc_lru_import(ffc_lru_t* h, const int64_t* keys_host, const int32_t* slots_host, int64_t n, void* stream);
 

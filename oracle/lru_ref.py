@@ -158,3 +158,21 @@ class LRU:
 
     def keys(self):
         return self._slot_of.keys()
+
+
+def ref_batch(ref, qpos, keys, journal, qlog=None):
+    """ffc.py:166-177 over the oracle LRU: returns rows, cols, hits, ones (set); updates qpos (a list) in place.
+    With ``qlog`` (a list), appends (slot, qpos before) per access, so that undoing the last m accesses restores
+    qpos by popping m entries."""
+    rows, cols, hits, ones = [], [], [], set()
+    for k in keys:
+        known = k in ref
+        s = ref.try_get(k) if journal else ref.get(k)
+        if qlog is not None:
+            qlog.append((s, qpos[s]))
+        if known:
+            rows.append(qpos[s]); ones.add(s); qpos[s] ^= 1
+        else:
+            rows.append(0); qpos[s] = 1
+        cols.append(s); hits.append(1 if known else 0)
+    return rows, cols, hits, ones

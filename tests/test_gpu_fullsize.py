@@ -1,6 +1,6 @@
 """Full-size (BASELINE.json C3: queue 1,048,576 x D=512, 1024 rows) checks through size-independent properties:
 the tcgen05 path against the fp64 check mode on the same state, rollback idempotence, gradient linearity, and the
-LRU's defining property (the resident set is the most recently used `capacity` distinct keys)."""
+LRU slot for slot against the oracle, with its defining property (the resident set is the most recently used `capacity` distinct keys)."""
 import numpy as np
 import pytest
 import torch
@@ -60,25 +60,57 @@ def test_bf16_vs_check_mode_full_size():
 
 
 def test_lru_full_size_property():
-    """After any access stream the resident set must be the `capacity` most recently used distinct keys, every key
-    maps to a unique slot, and view() agrees with the slots handed out."""
+    """The 2^20-slot LRU against the oracle, slot for slot: cols and rows of every pass, qpos, view() of every key of the pass,
+    and state_dict.  About 1.2 M accesses: random keys plus 1/16 keys homed in 48 crafted windows of the 2^17-window table, in
+    committed passes and journaled ones that are undone.  Then the defining property on the committed stream: the resident set is
+    the `capacity` most recently used distinct keys, every key maps to a unique slot.  The test also counts the home windows that
+    held more than 32 live keys (a chain into the next window) at the end of some pass, and requires at least one."""
     import ffc_b200
+    from oracle import lru_keys as K
+    from oracle.lru_ref import LRU as RefLRU
+    from oracle.lru_ref import ref_batch
     dev = torch.device('cuda')
     cap = 1 << 20
-    lru = ffc_b200.LRU(cap)
+    nwin = K.table_windows(cap)
+    lru = ffc_b200.LRU(cap, journal_capacity=1 << 17)
+    ref = RefLRU(cap)
+    qpos = torch.zeros(cap, dtype=torch.uint8, device=dev)
+    ref_qpos = [0] * cap
     rng = np.random.default_rng(0)
+    wins = rng.choice(nwin, size=48, replace=False)
+    crafted = np.array([k for w in wins for k in K.keys_in_window(int(w), nwin, 80, rng)], dtype=np.int64)
     n_batches, bs = 12, 1024 * 96
-    last_use = {}
-    t = 0
     stream = []
+    crowded = set()
     for b in range(n_batches):
         keys = rng.integers(0, 3 * cap, size=bs, dtype=np.int64)
-        stream.append(keys)
-        cols = lru.assign(torch.from_numpy(keys).to(dev))
-        got = lru.view_batch(torch.from_numpy(keys).to(dev))
-        # a key accessed in this batch can only be missing if it was evicted again later in the same batch: impossible
-        # here because a batch (98k keys) is far smaller than the capacity
-        assert torch.equal(got, cols) or bool(((got == cols) | (got >= 0)).all())
+        pick = rng.choice(bs, size=bs // 16, replace=False)
+        keys[pick] = rng.choice(crafted, size=bs // 16)
+        journal = b % 3 == 1
+        kl = keys.tolist()
+        kt = torch.from_numpy(keys).to(dev)
+        rows = torch.empty(bs, dtype=torch.int32, device=dev)
+        cols = lru.assign(kt, journal=journal, qpos=qpos, rows=rows)
+        qlog = []
+        r_rows, r_cols, _, _ = ref_batch(ref, ref_qpos, kl, journal, qlog)
+        assert np.array_equal(cols.cpu().numpy(), np.array(r_cols)), b
+        assert np.array_equal(rows.cpu().numpy(), np.array(r_rows)), b
+        got = lru.view_batch(kt).cpu().numpy()
+        assert np.array_equal(got, np.array([ref.view(k) for k in kl])), b
+        crowded.update(np.flatnonzero(K.home_window_counts(ref.keys(), nwin) > 32).tolist())
+        if journal:
+            lru.undo(-1, qpos)
+            ref.rollback_steps(len(qlog))
+            for s, q in reversed(qlog):
+                ref_qpos[s] = q
+            assert lru.journal_len == 0
+        else:
+            stream.append(keys)
+        if b in (4, n_batches - 1):
+            assert lru.state_dict() == ref.state_dict(), b
+            assert qpos.cpu().tolist() == ref_qpos, b
+    print(f'home windows that held more than 32 live keys at the end of some pass: {len(crowded)}')
+    assert len(crowded) > 0
     allk = np.concatenate(stream)
     # most recent occurrence index of every distinct key
     rev = allk[::-1]

@@ -7,6 +7,7 @@ import pytest
 import torch
 
 from oracle.lru_ref import LRU as RefLRU
+from oracle.lru_ref import ref_batch as _ref_batch
 
 pytestmark = pytest.mark.gpu
 
@@ -46,20 +47,6 @@ def test_reference_traces_scalar_api(golden_dir):
                 assert lru.cur_idx == op[3]
             n += 1
     assert n > 1000
-
-
-def _ref_batch(ref, qpos, keys, journal):
-    """ffc.py:166-177 over the oracle LRU: returns rows, cols, hits, ones(set)"""
-    rows, cols, hits, ones = [], [], [], set()
-    for k in keys:
-        known = k in ref
-        s = ref.try_get(k) if journal else ref.get(k)
-        if known:
-            rows.append(qpos[s]); ones.add(s); qpos[s] ^= 1
-        else:
-            rows.append(0); qpos[s] = 1
-        cols.append(s); hits.append(1 if known else 0)
-    return rows, cols, hits, ones
 
 
 @pytest.mark.parametrize('cap,universe,batch', [(1, 5, 7), (2, 6, 16), (7, 12, 16), (64, 90, 48), (64, 4000, 64),

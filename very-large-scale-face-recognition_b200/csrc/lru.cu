@@ -153,7 +153,8 @@ __global__ void __launch_bounds__(256) lru_lookup_kernel(const int64_t* __restri
   const int wid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (wid >= n) return;
   const int64_t key = keys[wid];
-  const int32_t s = ht_find_warp(ht_key, ht_slot, nwin, key, lane, nullptr);
+  // the sentinels would match an empty cell / a tombstone: never resident
+  const int32_t s = (key == KEY_EMPTY || key == KEY_TOMB) ? -1 : ht_find_warp(ht_key, ht_slot, nwin, key, lane, nullptr);
   if (lane == 0) out[wid] = s;
 }
 
@@ -419,8 +420,10 @@ __device__ bool resolve_chunk(const ResolveArgs& a, ResolveSmem& S) {
   if (tid == 0 && a.ones_list) S.ones0 = *reinterpret_cast<volatile int32_t*>(a.n_ones);
   int64_t key = 0;
   int32_t s0 = -1;
+  bool reserved = false;
   if (tid < n) {
     key = a.keys[tid];
+    reserved = (key == KEY_EMPTY || key == KEY_TOMB);
     s0 = a.s0[tid];
     S.pkey[tid] = key;
     const int fs = cur0 + tid;
@@ -440,7 +443,11 @@ __device__ bool resolve_chunk(const ResolveArgs& a, ResolveSmem& S) {
     S.cur = cur0;
     S.err = 0;
   }
-  __syncthreads();
+  // a reserved key is neither a hit nor a miss: refuse the chunk before it changes anything (its s0 is meaningless)
+  if (__syncthreads_or(reserved)) {
+    if (tid == 0) st->err = 5;
+    return false;
+  }
 
   // R1: dedupe batch keys -> first occurrence -> node ids
   int mycell = -1;
@@ -659,6 +666,11 @@ __device__ bool resolve_chunk(const ResolveArgs& a, ResolveSmem& S) {
 // chunks cannot run side by side).  The table lookups of chunk 0 come from lru_lookup_kernel (many CTAs, launched just before);
 // later chunks depend on the inserts / evictions of the earlier ones, so the CTA looks their keys up itself (one warp per key).
 // With a device-side key count (sharded callers) the walk stops at clamp(*n_dev - n_base, 0, n): no empty launches.
+// Not inlined: inlined, the error path alone adds 24 B of spills to the resolve kernel (64 registers at 1 024 threads).
+__device__ __noinline__ void clear_cols(int32_t* cols, int n) {
+  for (int i = threadIdx.x; i < n; i += NT) cols[i] = -1;
+}
+
 __global__ void __launch_bounds__(NT, 1) lru_resolve_kernel(const ResolveArgs a_in) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   ResolveSmem& S = *reinterpret_cast<ResolveSmem*>(smem_raw);
@@ -683,7 +695,10 @@ __global__ void __launch_bounds__(NT, 1) lru_resolve_kernel(const ResolveArgs a_
       }
       __syncthreads();
     }
-    if (!resolve_chunk(a, S)) return;
+    if (!resolve_chunk(a, S)) {   // device error: no slot for the refused chunk and the rest, so consumers skip those positions
+      clear_cols(a.cols_out, n_total - base);
+      return;
+    }
   }
 }
 
@@ -894,7 +909,8 @@ static int lru_check_err(ffc_lru* h, cudaStream_t s) {
   FFC_CUDA(cudaMemcpyAsync(&err, &h->st->err, sizeof(err), cudaMemcpyDeviceToHost, s));
   FFC_CUDA(cudaStreamSynchronize(s));
   if (err) {
-    set_error("device LRU error flag %d (1=ring full, 2=journal full, 3=empty cache with zero capacity, 4=scan)", err);
+    set_error("device LRU error flag %d (1=ring full, 2=journal full, 3=empty cache with zero capacity, 4=scan, 5=reserved key); "
+              "the cache state is unspecified until clear() or restore()", err);
     return FFC_ERR_STATE;
   }
   return FFC_OK;
@@ -1071,7 +1087,8 @@ extern "C" int ffc_lru_size(ffc_lru_t* h, int64_t* cur_idx_out, int64_t* journal
   FFC_CUDA(cudaMemcpyAsync(&st, h->st, sizeof(st), cudaMemcpyDeviceToHost, s));
   FFC_CUDA(cudaStreamSynchronize(s));
   if (st.err) {
-    set_error("device LRU error flag %d (1=ring full, 2=journal full, 3=empty cache, 4=scan)", st.err);
+    set_error("device LRU error flag %d (1=ring full, 2=journal full, 3=empty cache, 4=scan, 5=reserved key); "
+              "the cache state is unspecified until clear() or restore()", st.err);
     return FFC_ERR_STATE;
   }
   if (cur_idx_out) *cur_idx_out = st.cur_idx;
@@ -1119,10 +1136,12 @@ extern "C" int ffc_lru_import(ffc_lru_t* h, const int64_t* keys_host, const int3
   FFC_REQUIRE(h && (n == 0 || (keys_host && slots_host)), "ffc_lru_import: NULL argument");
   FFC_REQUIRE(n >= 0 && n <= h->cap, "ffc_lru_import: %lld pairs exceed capacity %lld", (long long)n, (long long)h->cap);
   cudaStream_t s = (cudaStream_t)stream;
-  int64_t cur = 0;
-  int rc = ffc_lru_size(h, &cur, nullptr, s);
-  if (rc) return rc;
-  FFC_REQUIRE(cur == 0, "ffc_lru_import: cache not empty (cur_idx=%lld); lru.py:115 asserts cur_idx == 0", (long long)cur);
+  LruState st;
+  FFC_CUDA(cudaMemcpyAsync(&st, h->st, sizeof(st), cudaMemcpyDeviceToHost, s));
+  FFC_CUDA(cudaStreamSynchronize(s));
+  // a cache whose error flag is set holds an unspecified state: restoring over it is how it recovers
+  FFC_REQUIRE(st.err != 0 || st.cur_idx == 0, "ffc_lru_import: cache not empty (cur_idx=%lld); lru.py:115 asserts cur_idx == 0",
+              (long long)st.cur_idx);
   std::vector<int64_t> skey(n), spos(n);
   std::vector<int32_t> ring(n);
   std::vector<char> seen(n, 0);
@@ -1140,7 +1159,7 @@ extern "C" int ffc_lru_import(ffc_lru_t* h, const int64_t* keys_host, const int3
     std::sort(sorted.begin(), sorted.end());
     FFC_REQUIRE(std::adjacent_find(sorted.begin(), sorted.end()) == sorted.end(), "ffc_lru_import: duplicate key");
   }
-  rc = ffc_lru_clear(h, s);
+  int rc = ffc_lru_clear(h, s);
   if (rc) return rc;
   if (n > 0) {
     FFC_CUDA(cudaMemcpyAsync(h->slot_key, skey.data(), n * sizeof(int64_t), cudaMemcpyHostToDevice, s));
