@@ -172,7 +172,8 @@ __global__ void __launch_bounds__(128) head_target_kernel(const float* __restric
 // Everything a pass needs before its sweep, in ONE launch (block b: probe row b and/or side row b):
 //   row part   (b < n_rows): target column / position in `ones` / outlier flag / n_pos, n_out counts (head_prep_rows_kernel),
 //                            bf16 copy of the probe row (head_p_to_bf16_kernel), target cosines (head_target_kernel)
-//   side part  (b < ceil128(n_ones)): gathered `ones` rows of queue[0] and queue[1] (head_gather_side_kernel)
+//   side part  (rows j < min(ceil128(n_ones), max_rows), j = b, b + gridDim.x, ...): gathered `ones` rows of queue[0] and queue[1]
+//              (head_gather_side_kernel)
 // counts[2][2] is double-buffered by pass parity: block 0 clears the other parity's pair for the next pass (no memset launch).
 template <bool BF16>
 __global__ void __launch_bounds__(128) head_prep_fused_kernel(const float* __restrict__ P, __nv_bfloat16* __restrict__ P16, const int32_t* __restrict__ label,
@@ -253,9 +254,10 @@ __global__ void __launch_bounds__(128) head_prep_fused_kernel(const float* __res
       }
     }
   }
-  // side matrices: W_side0[j] = queue[0][ones[j]], W_side1[j] = queue[1][ones[j]], zero padded to the 128-row tile
-  if (b < ((no + 127) & ~127) && b < max_rows) {
-    const int j = b;
+  // side matrices: W_side0[j] = queue[0][ones[j]], W_side1[j] = queue[1][ones[j]], zero padded to the 128-row tile.  Grid-stride: the
+  // grid is sized by the probe rows, and a C-ABI caller may pass more `ones` slots than that (up to max_rows).
+  const int n_side = min((no + 127) & ~127, max_rows);
+  for (int j = b; j < n_side; j += gridDim.x) {
     const bool live = j < no;
     const int64_t slot = live ? ones_list[j] : 0;
     for (int r = 0; r < 2; ++r) {
@@ -1370,6 +1372,9 @@ static int head_sweep_impl(ffc_head_t* h, const ffc_head_pass* in, const ffc_hea
   a.n_cols_dev = in->n_ones;
   a.tcol = h->tpos;
   a.cmask = nullptr;
+  // Without the main sweep's shared threshold: side 0 would raise it to ITS k-th, and side 1 (merged with the main list for loss 2, not
+  // with side 0) would then drop the queue[1] candidates between the main k-th and that.  The side lists are complete, as in the merged launch.
+  a.kth_shared = nullptr;
   for (int l = 0; l < 2; ++l) {
     a.W_f32 = h->side_f32 + (int64_t)l * c.max_rows * D;
     a.W_bf16 = h->side_bf16 + (int64_t)l * c.max_rows * D;

@@ -30,7 +30,8 @@ struct SweepArgs {
   const uint8_t* is_out;         // [n_rows] 1 if the row takes part in the hard-negative top-k
   const int32_t* row_map;        // optional [n_rows]: sweep position -> probe row, hard-negative-only rows last (CTA-pair tcgen05 kernel; NULL = identity)
   const int32_t* n_pos_dev;      // ... and the number of rows in front of them (device side)
-  int32_t* kth_shared;           // [n_rows] zero-initialised scratch: threshold shared by the column chunks (tcgen05 path; never NULL there)
+  int32_t* kth_shared;           // [n_rows] zero-initialised scratch: threshold shared by the column chunks of the main sweep (tcgen05 path;
+                                 // NULL = none: the side sweeps launched on their own)
   float scale;                   // s
   float fixed_max;               // M
   int sv;                        // SV transform enabled

@@ -392,7 +392,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1)
         // has seen so far is a lower bound of the row's final k-th, so nothing at or below it can enter the merged top-k.  Each
         // item publishes its own k-th (atomicMax on the integer key) and picks the maximum up at every tile: the candidate rate
         // of an item falls as if it had seen all chunks' columns.  Main sweep only (the side sets merge per loss).
-        int32_t* kshare = (sidx == 0 && outl) ? prm.kth_shared + row : nullptr;
+        int32_t* kshare = (sidx == 0 && outl && prm.kth_shared) ? prm.kth_shared + row : nullptr;
         int kfloor = 0, kpub = 0;
         float pthr = __uint_as_float(__float_as_uint(ex2f(-b2)) & 0xffff0000u);    // p~ of cosine 0, rounded down to bf16
         if (!dbg_noS) {
@@ -447,7 +447,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1)
               }
             }
           }
-          if (outl) {
+          if (kshare) {
             if (kth > 0) {
               atomicMax(kshare, kth);
               kpub = kth;

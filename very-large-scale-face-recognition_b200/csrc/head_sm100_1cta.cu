@@ -212,7 +212,7 @@ __global__ void __launch_bounds__(NTHREADS, 1)
     }
     int kth = 0;
     uint32_t* scan_stage = reinterpret_cast<uint32_t*>(sW + Sh::SLOTS * Sh::TILE_BYTES) + (warp - 4) * 32;   // 128 bytes per epilogue warp
-    int32_t* kshare = (sidx == 0 && outl) ? prm.kth_shared + row : nullptr;      // threshold shared by the column chunks of a row (see head_sm100.cu)
+    int32_t* kshare = (sidx == 0 && outl && prm.kth_shared) ? prm.kth_shared + row : nullptr;      // threshold shared by the column chunks of a row (see head_sm100.cu)
     int kfloor = 0, kpub = 0;
     float pthr = __uint_as_float(__float_as_uint(ex2f(-b2)) & 0xffff0000u);
     const uint32_t lane_base = tmem_base + ((uint32_t)(q4 * 32) << 16);
